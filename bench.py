@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MCMC chain-steps/s (and ESS/s) of the fused Metropolis kernel on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, NCCL)
 
 A "step" is ONE launch of the fused kernel advancing every chain of the batch by `--mcmc-steps`
@@ -19,6 +19,13 @@ collective; one all-reduce of pooled moments/counters at the end (inside the tim
 
 `--impl reference` times the CPU restatement of the reference's sampler (oracle/, NumPy; the
 reference itself is pure Python + NumPy and cannot travel to the GPU box) on all host cores.
+
+`--dump-outputs DIR` writes what the last timed launch of the main workload returned, as float64 .npy files:
+samples (the recorded states, [chains, mcmc_steps, 3]), u and phi (the final state and Phi of every chain),
+model_state (Lorenz only: the carried initial condition) and pooled (the all-reduced moments and counters).
+The inputs are seeded, so two builds run with the same arguments can be compared array by array.  Above 64 MB
+a fixed, seeded subset of the chains is written, with their global ids in chain_index.  With several GPUs,
+rank 0 writes its own chains and the global pooled moments.
 """
 import argparse
 import json
@@ -48,6 +55,7 @@ WORKLOADS = {
     "lorenz_rw": dict(model="lorenz", chains=4096, mcmc_steps=128, delta=0.125, T=20.0),
 }
 SHORT_LAUNCH_STEPS = 200
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
 
 
 # ------------------------------------------------------------------------------------------------
@@ -270,6 +278,33 @@ def algorithmic_flops(wl, work_a, work_b):
     return 3444.0 * (work_a + work_b) + 48.0 * work_a
 
 
+def last_step_outputs(chains, trace, pooled):
+    """Host copies of what the last launch returned (see --dump-outputs).  When the per-chain arrays do not fit
+    in DUMP_LIMIT_BYTES, a subset of the chains drawn with a fixed seed is kept."""
+    import torch
+    per_chain = dict(samples=trace, u=chains.u, phi=chains.phi)
+    if chains.model_state is not None:
+        per_chain["model_state"] = chains.model_state
+    out = {}
+    chain_bytes = sum(t[0].numel() * t.element_size() for t in per_chain.values())
+    room = DUMP_LIMIT_BYTES - pooled.numel() * pooled.element_size() - 4096     # 4096: the .npy headers
+    if chains.n * chain_bytes > room:
+        idx = np.sort(np.random.default_rng(0).choice(chains.n, room // (chain_bytes + 8), replace=False))
+        sel = torch.as_tensor(idx, device=trace.device)
+        per_chain = {k: t.index_select(0, sel) for k, t in per_chain.items()}
+        out["chain_index"] = (idx + chains.chain_offset).astype(np.float64)
+    out.update({k: t.cpu().numpy() for k, t in per_chain.items()})
+    out["pooled"] = pooled.cpu().numpy()
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype == np.float64, (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def emit(line, out_fd):
     os.write(out_fd, (json.dumps(line) + "\n").encode())
 
@@ -292,7 +327,13 @@ def main():
     ap.add_argument("--burn-in", type=int, default=1500, help="untimed Metropolis steps before warm-up (Burgers)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary workload lines")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the arrays the last timed launch returned to DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     wl = dict(WORKLOADS[args.workload])
     if args.chains:
         wl["chains"] = args.chains
@@ -319,7 +360,7 @@ def main():
     sm_ghz = torch.cuda.get_device_properties(dev).clock_rate / 1e6 if hasattr(torch.cuda.get_device_properties(dev), "clock_rate") else 1.965
     nominal_fp64 = n_sm * 64 * 2 * 1.965e9 / 1e12      # 64 DFMA lanes per SM per clock at clocks.max.sm
 
-    def measure(wl, K, W, with_e2e=True, trace_chains=64, burn_in=0, start=None):
+    def measure(wl, K, W, with_e2e=True, trace_chains=64, burn_in=0, start=None, dump=False):
         B, S = wl["chains"], wl["mcmc_steps"]
         pot, proposer, accepter, u0 = build_problem(M, wl, wl.get("numerics", args.numerics))
         sampler = M.MCMCSampler(proposer, accepter, np.random.default_rng(2))
@@ -374,6 +415,7 @@ def main():
         t_wall = time.perf_counter() - t_wall0
         sampler_clk.stop_flag = True
         sampler_clk.join()
+        outputs = last_step_outputs(chains, trace, pooled) if dump else None
         kern_ms = [a.elapsed_time(b) for a, b in ev[:K]]
         red_ms = ev[K][0].elapsed_time(ev[K][1])
         pool_ms = ev[K][0].elapsed_time(ev_mid)
@@ -407,7 +449,8 @@ def main():
                    ess_per_chain=ess_per_chain, clocks=sampler_clk.summary(), launches=chains.launches - launches0,
                    pooled=pooled.cpu().numpy(), wall_s=t_wall, nonfinite=int(dc_all[4]),
                    mean_work_per_solve=dc_all[2] / max(dc_all[3], 1)
-                   if wl["model"] == "burgers" else (dc_all[2] + dc_all[3]) / max(2 * dc_all[0], 1))
+                   if wl["model"] == "burgers" else (dc_all[2] + dc_all[3]) / max(2 * dc_all[0], 1),
+                   outputs=outputs)
         if with_e2e:
             # end to end through the public API with HOST buffers: numpy u_0 (and Phi(u_0), known from the run that
             # produced it) in, numpy samples out.  (1) MCMCSampler.run: torch-managed pinned staging;
@@ -496,7 +539,10 @@ def main():
         if wl['N'] >= 1024:
             burn_in = min(burn_in, 200)        # a solve costs ~30 MFLOP here: keep the untimed part short
     args.burn_in = burn_in
-    res = measure(wl, args.steps, max(args.warmup, 3), burn_in=burn_in, start=start)
+    res = measure(wl, args.steps, max(args.warmup, 3), burn_in=burn_in, start=start,
+                  dump=bool(args.dump_outputs) and rank == 0)
+    if res["outputs"] is not None:
+        write_outputs(args.dump_outputs, res["outputs"])
     extra = {}
     cold = None
     if not args.no_extra and args.workload == "burgers_pcn_256":
