@@ -19,10 +19,6 @@ UNITS = ([("engine", "engine.cu", [])]
          + [("burgers_cpl%d_%s" % (c, "fused" if num else "exact"), "burgers_inst.cu",
              ["-DIPMCMC_TU_CPL=%d" % c, "-DIPMCMC_TU_NUM=%d" % num]) for c in (32, 16, 8, 7, 4, 2, 1) for num in (1, 0)]
          + [("burgers_cpl0", "burgers_inst.cu", ["-DIPMCMC_TU_CPL=0"])])
-SOURCES = ["engine.cu", "burgers_inst.cu"]
-HEADERS = ["common.cuh", "philox.cuh", "burgers.cuh", "burgers_kernels.cuh", "burgers_team.cuh", "burgers_launch.cuh",
-           "burgers_launch_impl.cuh", "lorenz.cuh", "lorenz_kernels.cuh", "sampler.cuh",
-           os.path.join("..", "..", "include", "ipmcmc.h")]
 # No --split-compile: with it ptxas' output is not reproducible (the schedule of the Burgers time-step loop
 # came out in one of two variants, 15 % apart in throughput, from one build of the same source to the next).
 CFLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
@@ -30,7 +26,8 @@ CFLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fm
 NVCC_FLAGS = CFLAGS      # (name kept for tools/)
 
 
-# headers each kind of unit includes (a unit is recompiled when its object is older than any of them)
+# headers each kind of unit includes: a unit is recompiled when its object, and the library is relinked when it,
+# is older than the unit's source or any of them
 _COMMON = ["common.cuh", "philox.cuh", "sampler.cuh", "sched.cuh", "burgers.cuh", "burgers_launch.cuh",
            os.path.join("..", "..", "include", "ipmcmc.h")]
 DEPS = {"engine.cu": _COMMON + ["lorenz.cuh", "lorenz_kernels.cuh"],
@@ -54,7 +51,7 @@ def _stale():
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    return any(_mtime(f) > t for f in SOURCES + HEADERS)
+    return any(_mtime(f) > t for src, deps in DEPS.items() for f in [src] + deps)
 
 
 def compile_units(out_lib, extra_flags=(), obj_dir=None, verbose=False, force=True):

@@ -9,27 +9,13 @@
 #include "sched.cuh"
 
 // Register budget of the static chain kernel: 128 registers (2 CTAs of 256 threads per SM) up to 8 cells
-// per lane, 255 from 16 cells per lane on, where 128 spill the state (measured: engine.cu,
+// per lane, 255 from 16 cells per lane on, where 128 spill the state (measured: burgers_launch_impl.cuh,
 // burgers_launch_chain_queue).
 #ifndef IPMCMC_CHAIN_MINB
 #define IPMCMC_CHAIN_MINB(CPL) ((CPL) >= 16 ? 1 : 2)
 #endif
 
 namespace ipmcmc {
-
-// Developer instrumentation (-DIPMCMC_PROF=1, tools/overhead_probe.py): cycles per section of a work
-// item, summed over all warps by lane 0.  Not compiled into the product library.
-#ifndef IPMCMC_PROF
-#define IPMCMC_PROF 0
-#endif
-#if IPMCMC_PROF
-static __device__ unsigned long long g_prof[16];
-#define PROF_T(var) const long long var = clock64()
-#define PROF_ADD(slot, a, b) do { if (lane_id() == 0) atomicAdd(&g_prof[slot], (unsigned long long)((b) - (a))); } while (0)
-#else
-#define PROF_T(var)
-#define PROF_ADD(slot, a, b)
-#endif
 
 // shared memory layout per warp: state[N] | G[MAX_OBS] | r2[MAX_OBS]
 __host__ __device__ inline size_t burgers_smem_bytes(int N, int warps = 1) {
@@ -84,6 +70,24 @@ __device__ IPMCMC_PHI_INLINE double burgers_phi(const BurgersDev &B, double ui, 
     return W.capped ? nan("") : phi;
 }
 
+// Outputs of forward evaluation c (null pointers are skipped): G and the end state from shared memory,
+// Phi and the work.  Thread t of the nt threads that evaluated it (a warp or a team) writes every nt-th value.
+__device__ __forceinline__ void burgers_store_forward(const BurgersDev &B, long long c, const double *Gs,
+                                                      const double *state, double ph, int n_fv, double *G, double *phi,
+                                                      double *state_out, long long *work, int t, int nt) {
+    if (G)
+        for (int i = t; i < B.pot.q; i += nt) G[c * B.pot.q + i] = Gs[i];
+    if (state_out)
+        for (int i = t; i < B.N; i += nt) state_out[c * B.N + i] = state[i];
+    if (t == 0) {
+        if (phi) phi[c] = ph;
+        if (work) {
+            work[2 * c] = n_fv;
+            work[2 * c + 1] = 0;
+        }
+    }
+}
+
 template <int CPL, int NUMERICS, bool PADDED>
 __global__ void __launch_bounds__(256) burgers_forward_kernel(const __grid_constant__ BurgersDev B, long long n,
                                                               const double *__restrict__ u, double *__restrict__ G,
@@ -98,17 +102,7 @@ __global__ void __launch_bounds__(256) burgers_forward_kernel(const __grid_const
         const double ui = (lane < B.d) ? u[c * B.d + lane] : 0.0;
         int n_fv;
         const double ph = burgers_phi<CPL, NUMERICS, PADDED>(B, ui, state, Gs, r2, lane, n_fv);
-        if (G)
-            for (int i = lane; i < B.pot.q; i += 32) G[c * B.pot.q + i] = Gs[i];
-        if (state_out)
-            for (int i = lane; i < B.N; i += 32) state_out[c * B.N + i] = state[i];
-        if (lane == 0) {
-            if (phi) phi[c] = ph;
-            if (work) {
-                work[2 * c] = n_fv;
-                work[2 * c + 1] = 0;
-            }
-        }
+        burgers_store_forward(B, c, Gs, state, ph, n_fv, G, phi, state_out, work, lane, 32);
         __syncwarp();
     }
 }
@@ -191,15 +185,75 @@ __device__ IPMCMC_STEP_INLINE void metropolis_step(const SamplerDev &S, const Ch
     }
 }
 
+// Chain c's registers from global memory (ld_state<QUEUE>).  On the chain's first launch Phi(u_0) is not
+// known yet (NaN) and is solved for with `phi_of`.  `team`: every warp of the CTA runs this for the same
+// chain, and all must have read the state before warp 0 may overwrite it (burgers_store_chain).
+template <bool QUEUE, class PhiOf>
+__device__ __forceinline__ ChainRegs burgers_load_chain(const SamplerDev &S, const ChainBufDev &C, const Group &Gp,
+                                                        long long c, const PhiOf &phi_of, bool team) {
+    const int lane = Gp.lane, d = S.d;
+    ChainRegs R;
+    R.ui = (lane < d) ? ld_state<QUEUE>(C.u + c * d + lane) : 0.0;
+    R.phi_u = ld_state<QUEUE>(C.phi + c);
+#pragma unroll
+    for (int k = 0; k < CNT_N; ++k) R.cnt[k] = 0;
+    if (team) __syncthreads();
+    if (isnan(R.phi_u)) {
+        int n_fv;
+        R.phi_u = phi_of(R.ui, n_fv);
+        R.cnt[CNT_WORK_A] += n_fv;
+        R.cnt[CNT_WORK_B] += 1;
+    }
+    R.reg_u = (S.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser(S, Gp, R.ui) : 0.0;
+    R.mom = Welford{ld_state<QUEUE>(C.mom_count + c), (lane < d) ? ld_state<QUEUE>(C.mom_mean + c * d + lane) : 0.0,
+                    (lane < d) ? ld_state<QUEUE>(C.mom_m2 + c * d + lane) : 0.0};
+    return R;
+}
+
+// Chain c's registers back to global memory; the counters accumulate over launches.  A chain belongs to
+// one warp (or team) at a time, so their read-modify-write needs no atomic, under the queue too (sched.cuh).
+template <bool QUEUE>
+__device__ __forceinline__ void burgers_store_chain(const SamplerDev &S, const ChainBufDev &C, int lane, long long c,
+                                                    const ChainRegs &R) {
+    const int d = S.d;
+    if (lane < d) {
+        st_state<QUEUE>(C.u + c * d + lane, R.ui);
+        st_state<QUEUE>(C.mom_mean + c * d + lane, R.mom.mean);
+        st_state<QUEUE>(C.mom_m2 + c * d + lane, R.mom.m2);
+    }
+    if (lane == 0) {
+        st_state<QUEUE>(C.phi + c, R.phi_u);
+        st_state<QUEUE>(C.mom_count + c, R.mom.count);
+#pragma unroll
+        for (int k = 0; k < CNT_N; ++k)
+            st_state<QUEUE>(C.counters + c * CNT_N + k, ld_state<QUEUE>(C.counters + c * CNT_N + k) + R.cnt[k]);
+    }
+}
+
+// `phi_of` of the one-warp solver.  A functor and not a lambda: with three call sites (first launch, Phi(u),
+// Phi(v)) NVVM outlined a lambda's call operator, and with it the whole solve (see burgers_phi).
 template <int CPL, int NUMERICS, bool PADDED>
-__device__ IPMCMC_STEP_INLINE void burgers_metropolis_step(const BurgersDev &B, const SamplerDev &S, const ChainBufDev &C,
-                                                        const Group &Gp, long long c, long long cg, long long s,
-                                                        long long n_steps, double *state, double *Gs, double *r2,
-                                                        ChainRegs &R) {
+struct BurgersPhiOf {
+    const BurgersDev &B;
+    double *state, *Gs, *r2;
+    int lane;
+    __device__ __forceinline__ double operator()(double ui, int &n_fv) const {
+        return burgers_phi<CPL, NUMERICS, PADDED>(B, ui, state, Gs, r2, lane, n_fv);
+    }
+};
+
+// Metropolis steps [s0, s1) of the launch for chain c on one warp: load the chain state, step, store it back.
+template <int CPL, int NUMERICS, bool PADDED, bool QUEUE>
+__device__ __forceinline__ void burgers_advance_chain(const BurgersDev &B, const SamplerDev &S, const ChainBufDev &C,
+                                                      const Group &Gp, long long c, long long s0, long long s1,
+                                                      long long n_steps, double *state, double *Gs, double *r2) {
     const int lane = Gp.lane;
-    metropolis_step(S, C, Gp, c, cg, s, n_steps, R,
-                    [&](double ui, int &n_fv) { return burgers_phi<CPL, NUMERICS, PADDED>(B, ui, state, Gs, r2, lane, n_fv); },
-                    true);
+    const long long cg = S.chain_offset + c;
+    const BurgersPhiOf<CPL, NUMERICS, PADDED> phi_of{B, state, Gs, r2, lane};
+    ChainRegs R = burgers_load_chain<QUEUE>(S, C, Gp, c, phi_of, false);
+    for (long long s = s0; s < s1; ++s) metropolis_step(S, C, Gp, c, cg, s, n_steps, R, phi_of, true);
+    burgers_store_chain<QUEUE>(S, C, lane, c, R);
+    __syncwarp();
 }
 
 // W warps per CTA, one chain per warp.  Warps never synchronise with each other; the CTA shape
@@ -213,48 +267,18 @@ __global__ void __launch_bounds__(256, IPMCMC_CHAIN_MINB(CPL)) burgers_chain_ker
     const int warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
     double *smem = smem_all + (size_t)warp * (B.N + 2 * IPMCMC_MAX_OBS);
     double *state = smem, *Gs = smem + B.N, *r2 = Gs + IPMCMC_MAX_OBS;
-    const int lane = lane_id();
-    const Group Gp{0, 32, lane, FULL};
-    const int d = S.d;
+    const Group Gp{0, 32, lane_id(), FULL};
     const long long n_slots = C.slot_chain ? (long long)C.n_slots : n_chains;
     for (long long slot = (long long)blockIdx.x * wpc + warp; slot < n_slots; slot += (long long)gridDim.x * wpc) {
         const long long c = C.slot_chain ? (long long)C.slot_chain[slot] : slot;
         if (c < 0 || c >= n_chains) continue;
-        const long long cg = S.chain_offset + c;
-        ChainRegs R;
-        R.ui = (lane < d) ? C.u[c * d + lane] : 0.0;
-        R.phi_u = C.phi[c];
-#pragma unroll
-        for (int k = 0; k < CNT_N; ++k) R.cnt[k] = 0;
-        if (isnan(R.phi_u)) {  // first launch: Phi(u_0) not known yet
-            int n_fv;
-            R.phi_u = burgers_phi<CPL, NUMERICS, PADDED>(B, R.ui, state, Gs, r2, lane, n_fv);
-            R.cnt[CNT_WORK_A] += n_fv;
-            R.cnt[CNT_WORK_B] += 1;
-        }
-        R.reg_u = (S.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser(S, Gp, R.ui) : 0.0;
-        R.mom = Welford{C.mom_count[c], (lane < d) ? C.mom_mean[c * d + lane] : 0.0,
-                        (lane < d) ? C.mom_m2[c * d + lane] : 0.0};
-        for (long long s = 0; s < n_steps; ++s)
-            burgers_metropolis_step<CPL, NUMERICS, PADDED>(B, S, C, Gp, c, cg, s, n_steps, state, Gs, r2, R);
-        // write back
-        if (lane < d) {
-            C.u[c * d + lane] = R.ui;
-            C.mom_mean[c * d + lane] = R.mom.mean;
-            C.mom_m2[c * d + lane] = R.mom.m2;
-        }
-        if (lane == 0) {
-            C.phi[c] = R.phi_u;
-            C.mom_count[c] = R.mom.count;
-#pragma unroll
-            for (int k = 0; k < CNT_N; ++k) C.counters[c * CNT_N + k] += R.cnt[k];
-        }
-        __syncwarp();
+        burgers_advance_chain<CPL, NUMERICS, PADDED, false>(B, S, C, Gp, c, 0, n_steps, n_steps, state, Gs, r2);
     }
 }
 
+// Dynamic step scheduler (sched.cuh): the work unit is a chain, an item is `chunk` Metropolis steps of it.
 // MINB: register budget, 2 = 128 registers (16 warps per SM), 1 = 255 registers; chosen by the number of
-// cells per lane in burgers_launch_chain_queue (engine.cu), where the measurements are quoted.
+// cells per lane in burgers_launch_chain_queue (burgers_launch_impl.cuh), where the measurements are quoted.
 template <int CPL, int NUMERICS, bool PADDED, int MINB>
 __global__ void __launch_bounds__(256, MINB) burgers_chain_queue_kernel(
     const __grid_constant__ BurgersDev B, const __grid_constant__ SamplerDev S, const __grid_constant__ ChainBufDev C,
@@ -265,78 +289,9 @@ __global__ void __launch_bounds__(256, MINB) burgers_chain_queue_kernel(
     double *state = smem, *Gs = smem + B.N, *r2 = Gs + IPMCMC_MAX_OBS;
     const int lane = lane_id();
     const Group Gp{0, 32, lane, FULL};
-    const int d = S.d;
-    SchedView Q(C.sched, n_chains);
-    const unsigned long long cap = (unsigned long long)Q.cap;
-    const long long items_per_chain = (n_steps + chunk - 1) / chunk;
-    const unsigned long long total = (unsigned long long)n_chains * (unsigned long long)items_per_chain;
-    while (true) {
-        // ---- take a ticket, wait for its ring slot to be filled, consume it
-        PROF_T(t0);
-        unsigned long long idx = 0;
-        if (lane == 0) idx = atomicAdd(Q.head, 1ull);
-        idx = __shfl_sync(FULL, idx, 0);
-        if (idx >= total) break;
-        unsigned long long *slot = Q.ring + idx % cap;
-        const unsigned long long want = idx / cap + 1;
-        const unsigned long long e = spin_until(slot, lane, [want](unsigned long long v) { return (v >> 32) == want; });
-        // mark the slot consumed: ordered after our own read of it (same address), nothing to publish
-        if (lane == 0) st_relaxed_u64(slot, 0ull);
-        __syncwarp();
-        const long long c = (long long)(e & 0xffffffffull), cg = S.chain_offset + c;
-        // ---- chain state from L2 (another SM may have written it: bypass L1)
-        const long long s0 = __ldcg(Q.progress + c);
-        ChainRegs R;
-        R.ui = (lane < d) ? __ldcg(C.u + c * d + lane) : 0.0;
-        R.phi_u = __ldcg(C.phi + c);
-#pragma unroll
-        for (int k = 0; k < CNT_N; ++k) R.cnt[k] = 0;
-        if (isnan(R.phi_u)) {  // first launch: Phi(u_0) not known yet
-            int n_fv;
-            R.phi_u = burgers_phi<CPL, NUMERICS, PADDED>(B, R.ui, state, Gs, r2, lane, n_fv);
-            R.cnt[CNT_WORK_A] += n_fv;
-            R.cnt[CNT_WORK_B] += 1;
-        }
-        R.reg_u = (S.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser(S, Gp, R.ui) : 0.0;
-        R.mom = Welford{__ldcg(C.mom_count + c), (lane < d) ? __ldcg(C.mom_mean + c * d + lane) : 0.0,
-                        (lane < d) ? __ldcg(C.mom_m2 + c * d + lane) : 0.0};
-        const long long s1 = (s0 + chunk < n_steps) ? s0 + chunk : n_steps;
-        PROF_T(t1);
-        for (long long s = s0; s < s1; ++s)
-            burgers_metropolis_step<CPL, NUMERICS, PADDED>(B, S, C, Gp, c, cg, s, n_steps, state, Gs, r2, R);
-        PROF_T(t2);
-        // ---- write back, then hand the chain to the next free warp.  The chain state is published by
-        // the release store of the ring entry (no separate fence): the other lanes' stores are ordered
-        // before it by __syncwarp (cumulativity).
-        if (lane < d) {
-            __stcg(C.u + c * d + lane, R.ui);
-            __stcg(C.mom_mean + c * d + lane, R.mom.mean);
-            __stcg(C.mom_m2 + c * d + lane, R.mom.m2);
-        }
-        if (lane == 0) {
-            __stcg(C.phi + c, R.phi_u);
-            __stcg(C.mom_count + c, R.mom.count);
-#pragma unroll
-            for (int k = 0; k < CNT_N; ++k) atomicAdd((unsigned long long *)(C.counters + c * CNT_N + k), (unsigned long long)R.cnt[k]);
-            __stcg(Q.progress + c, s1);
-        }
-        __syncwarp();
-        if (s1 < n_steps) {   // warp-uniform
-            unsigned long long t = 0;
-            if (lane == 0) t = atomicAdd(Q.tail, 1ull);
-            t = __shfl_sync(FULL, t, 0);
-            unsigned long long *pslot = Q.ring + t % cap;
-            spin_until(pslot, lane, [](unsigned long long v) { return v == 0ull; });   // previous lap consumed (cap = 2n: no wait in practice)
-            if (lane == 0) st_release_u64(pslot, ((t / cap + 1) << 32) | (unsigned long long)c);
-        }
-        __syncwarp();
-        PROF_T(t3);
-        PROF_ADD(0, t0, t3);
-        PROF_ADD(1, t0, t1);
-        PROF_ADD(6, t1, t2);
-        PROF_ADD(7, t2, t3);
-        PROF_ADD(8, 0, 1);
-    }
+    sched_serve(C.sched, n_chains, n_steps, chunk, lane, [&](long long c, long long s0, long long s1) {
+        burgers_advance_chain<CPL, NUMERICS, PADDED, true>(B, S, C, Gp, c, s0, s1, n_steps, state, Gs, r2);
+    });
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -408,17 +363,7 @@ __global__ void __launch_bounds__(128) burgers_wide_forward_kernel(const __grid_
         __syncwarp();
         int n_fv;
         const double ph = burgers_phi_wide<CPL, NUMERICS, PADDED>(B, x, par, state, Gs, r2, lane, n_fv);
-        if (G)
-            for (int i = lane; i < B.pot.q; i += 32) G[c * B.pot.q + i] = Gs[i];
-        if (state_out)
-            for (int i = lane; i < B.N; i += 32) state_out[c * B.N + i] = state[i];
-        if (lane == 0) {
-            if (phi) phi[c] = ph;
-            if (work) {
-                work[2 * c] = n_fv;
-                work[2 * c + 1] = 0;
-            }
-        }
+        burgers_store_forward(B, c, Gs, state, ph, n_fv, G, phi, state_out, work, lane, 32);
         __syncwarp();
     }
 }
@@ -573,17 +518,7 @@ __global__ void __launch_bounds__(32 * TM) burgers_team_forward_kernel(const __g
         const double ui = (lane < B.d) ? u[c * B.d + lane] : 0.0;
         int n_fv;
         const double ph = burgers_team_phi<CPL, NUMERICS, TM>(B, X, ui, state, Gs, r2, tw, lane, n_fv);
-        if (G && tw == 0)
-            for (int i = lane; i < B.pot.q; i += 32) G[c * B.pot.q + i] = Gs[i];
-        if (state_out)
-            for (int i = threadIdx.x; i < B.N; i += blockDim.x) state_out[c * B.N + i] = state[i];
-        if (threadIdx.x == 0) {
-            if (phi) phi[c] = ph;
-            if (work) {
-                work[2 * c] = n_fv;
-                work[2 * c + 1] = 0;
-            }
-        }
+        burgers_store_forward(B, c, Gs, state, ph, n_fv, G, phi, state_out, work, threadIdx.x, blockDim.x);
         __syncthreads();
     }
 }
@@ -599,42 +534,15 @@ __global__ void __launch_bounds__(32 * TM) burgers_team_chain_kernel(const __gri
     const int tw = threadIdx.x >> 5, lane = lane_id();
     const bool writer = tw == 0;  // all warps run the same Metropolis logic; warp 0 owns the global writes
     const Group Gp{0, 32, lane, FULL};
-    const int d = S.d;
     const auto phi_of = [&](double ui, int &n_fv) {
         return burgers_team_phi<CPL, NUMERICS, TM>(B, X, ui, state, Gs, r2, tw, lane, n_fv);
     };
     for (long long c = blockIdx.x; c < n_chains; c += gridDim.x) {
         const long long cg = S.chain_offset + c;
-        ChainRegs R;
-        R.ui = (lane < d) ? C.u[c * d + lane] : 0.0;
-        R.phi_u = C.phi[c];
-#pragma unroll
-        for (int k = 0; k < CNT_N; ++k) R.cnt[k] = 0;
-        __syncthreads();  // everyone has read the chain state before warp 0 may overwrite it at the end
-        if (isnan(R.phi_u)) {
-            int n_fv;
-            R.phi_u = phi_of(R.ui, n_fv);
-            R.cnt[CNT_WORK_A] += n_fv;
-            R.cnt[CNT_WORK_B] += 1;
-        }
-        R.reg_u = (S.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser(S, Gp, R.ui) : 0.0;
-        R.mom = Welford{C.mom_count[c], (lane < d) ? C.mom_mean[c * d + lane] : 0.0,
-                        (lane < d) ? C.mom_m2[c * d + lane] : 0.0};
+        ChainRegs R = burgers_load_chain<false>(S, C, Gp, c, phi_of, true);
         for (long long s = 0; s < n_steps; ++s) metropolis_step(S, C, Gp, c, cg, s, n_steps, R, phi_of, writer);
         __syncthreads();
-        if (writer) {
-            if (lane < d) {
-                C.u[c * d + lane] = R.ui;
-                C.mom_mean[c * d + lane] = R.mom.mean;
-                C.mom_m2[c * d + lane] = R.mom.m2;
-            }
-            if (lane == 0) {
-                C.phi[c] = R.phi_u;
-                C.mom_count[c] = R.mom.count;
-#pragma unroll
-                for (int k = 0; k < CNT_N; ++k) C.counters[c * CNT_N + k] += R.cnt[k];
-            }
-        }
+        if (writer) burgers_store_chain<false>(S, C, lane, c, R);
         __syncthreads();
     }
 }

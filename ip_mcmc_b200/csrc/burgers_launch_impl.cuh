@@ -16,7 +16,14 @@ namespace ipmcmc {
         if (e_ != cudaSuccess) return e_;             \
     } while (0)
 
-static inline int grid_for(long long n_blocks) { return (int)(n_blocks < 2147483647LL ? n_blocks : 2147483647LL); }
+// kern<<<grid, block, smem, st>>>(args...), after raising the kernel's dynamic shared-memory limit when
+// smem exceeds the 48 KB default.
+template <class... P, class... A>
+static cudaError_t launch(void (*kern)(P...), int grid, int block, size_t smem, cudaStream_t st, const A &...args) {
+    if (smem > 48 * 1024) IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, block, smem, st>>>(args...);
+    return cudaGetLastError();
+}
 
 template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_forward(const BurgersDev &b, long long n, const double *u, double *G, double *phi,
@@ -24,33 +31,24 @@ cudaError_t burgers_launch_forward(const BurgersDev &b, long long n, const doubl
     // one chain per warp; CTAs of 4 warps (one per SM sub-partition) unless the batch is tiny
     int wpc = n >= 4 * 148 ? 4 : 1;
     if (const char *e = getenv("IPMCMC_FWD_WPC")) wpc = atoi(e) > 0 && atoi(e) <= 8 ? atoi(e) : wpc;  // experiments
-    const size_t smem = burgers_smem_bytes(b.N, wpc);
-    auto kern = burgers_forward_kernel<CPL, NUM, PAD>;
-    if (smem > 48 * 1024) IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid_for((n + wpc - 1) / wpc), 32 * wpc, smem, st>>>(b, n, u, G, phi, state, work);
-    IPMCMC_CU(cudaGetLastError());
-    return cudaSuccess;
+    return launch(burgers_forward_kernel<CPL, NUM, PAD>, grid_for((n + wpc - 1) / wpc), 32 * wpc,
+                  burgers_smem_bytes(b.N, wpc), st, b, n, u, G, phi, state, work);
 }
 
 template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_chain(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,
                                 long long n_steps, int wpc, cudaStream_t st) {
-    const size_t smem = burgers_smem_bytes(b.N, wpc);
-    auto kern = burgers_chain_kernel<CPL, NUM, PAD>;
-    if (smem > 48 * 1024) IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const long long slots = C.slot_chain ? (long long)C.n_slots : n_chains;
-    kern<<<grid_for((slots + wpc - 1) / wpc), 32 * wpc, smem, st>>>(b, S, C, n_chains, n_steps);
-    IPMCMC_CU(cudaGetLastError());
-    return cudaSuccess;
+    return launch(burgers_chain_kernel<CPL, NUM, PAD>, grid_for((slots + wpc - 1) / wpc), 32 * wpc,
+                  burgers_smem_bytes(b.N, wpc), st, b, S, C, n_chains, n_steps);
 }
 
 // Dynamic step scheduler (burgers_chain_queue_kernel): persistent warps, one wave.
 template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_chain_queue(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,
                                       long long n_steps, int chunk, cudaStream_t st) {
-    int dev = 0, n_sm = 148;
-    IPMCMC_CU(cudaGetDevice(&dev));
-    IPMCMC_CU(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+    int n_sm = 148;
+    IPMCMC_CU(sm_count(n_sm));
     // small batches: one CTA of W = ceil(n / n_SM) warps per SM (warp w -> sub-partition w % 4);
     // large batches: as many 4-warp CTAs as are resident at once (register and shared-memory limits).
     // Register budget (measured on B200, DESIGN.md section 6; tools/ab_bench.sh): up to 8 cells per lane the 128-register
@@ -59,34 +57,26 @@ cudaError_t burgers_launch_chain_queue(const BurgersDev &b, const SamplerDev &S,
     // half the resident warps win by far (8192 x 1024: 81 % against 66 %; 88 % with the rotated loop, which
     // only fits the 255-register build at 32 cells per lane).
     int wpc, grid;
-    const bool small = n_chains <= 8LL * n_sm;
     constexpr int MINB = CPL >= 16 ? 1 : 2;
     auto kern = burgers_chain_queue_kernel<CPL, NUM, PAD, MINB>;
-    if (small) {
+    if (n_chains <= 8LL * n_sm) {
         wpc = (int)((n_chains + n_sm - 1) / n_sm);
         if (const char *e = getenv("IPMCMC_SCHED_WPC")) wpc = atoi(e) > 0 && atoi(e) <= 8 ? atoi(e) : wpc;  // experiments
         grid = (int)((n_chains + wpc - 1) / wpc);
         if (grid > n_sm) grid = n_sm;
         if (grid < n_sm && (long long)grid * wpc < n_chains) grid = n_sm;
     } else {
+        // 4 warps of at most 1024 cells: within the default 48 KB of shared memory
         wpc = 4;
-        grid = 0;
-    }
-    const size_t smem = burgers_smem_bytes(b.N, wpc);
-    if (smem > 48 * 1024) IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (grid == 0) {
         int per_sm = 0;
-        IPMCMC_CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 32 * wpc, smem));
+        IPMCMC_CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 32 * wpc, burgers_smem_bytes(b.N, wpc)));
         if (per_sm < 1) per_sm = 1;
         grid = per_sm * n_sm;
         const long long need = (n_chains + wpc - 1) / wpc;
         if (grid > need) grid = (int)need;
     }
-    sched_init_kernel<<<(unsigned)((2 * n_chains + 255) / 256 < 1184 ? (2 * n_chains + 255) / 256 : 1184), 256, 0, st>>>(C.sched, n_chains);
-    IPMCMC_CU(cudaGetLastError());
-    kern<<<grid, 32 * wpc, smem, st>>>(b, S, C, n_chains, n_steps, chunk);
-    IPMCMC_CU(cudaGetLastError());
-    return cudaSuccess;
+    IPMCMC_CU(sched_init(C.sched, n_chains, st));
+    return launch(kern, grid, 32 * wpc, burgers_smem_bytes(b.N, wpc), st, b, S, C, n_chains, n_steps, chunk);
 }
 
 // wide parameter vectors: 4 warps per CTA unless the shared memory of 4 does not fit
@@ -95,45 +85,29 @@ cudaError_t burgers_launch_wide_forward(const BurgersDev &b, long long n, const 
                                        double *state, long long *work, cudaStream_t st) {
     int wpc = n >= 4 * 148 ? 4 : 1;
     while (wpc > 1 && burgers_wide_smem_bytes(b.N, b.d, wpc) > 200 * 1024) wpc /= 2;
-    const size_t smem = burgers_wide_smem_bytes(b.N, b.d, wpc);
-    auto kern = burgers_wide_forward_kernel<CPL, NUM, PAD>;
-    if (smem > 48 * 1024) IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid_for((n + wpc - 1) / wpc), 32 * wpc, smem, st>>>(b, n, u, G, phi, state, work);
-    IPMCMC_CU(cudaGetLastError());
-    return cudaSuccess;
+    return launch(burgers_wide_forward_kernel<CPL, NUM, PAD>, grid_for((n + wpc - 1) / wpc), 32 * wpc,
+                  burgers_wide_smem_bytes(b.N, b.d, wpc), st, b, n, u, G, phi, state, work);
 }
 template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_wide_chain(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,
                                      long long n_steps, cudaStream_t st) {
     int wpc = n_chains >= 4 * 148 ? 4 : 1;
     while (wpc > 1 && burgers_wide_smem_bytes(b.N, S.d, wpc) > 200 * 1024) wpc /= 2;
-    const size_t smem = burgers_wide_smem_bytes(b.N, S.d, wpc);
-    auto kern = burgers_wide_chain_kernel<CPL, NUM, PAD>;
-    if (smem > 48 * 1024) IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid_for((n_chains + wpc - 1) / wpc), 32 * wpc, smem, st>>>(b, S, C, n_chains, n_steps);
-    IPMCMC_CU(cudaGetLastError());
-    return cudaSuccess;
+    return launch(burgers_wide_chain_kernel<CPL, NUM, PAD>, grid_for((n_chains + wpc - 1) / wpc), 32 * wpc,
+                  burgers_wide_smem_bytes(b.N, S.d, wpc), st, b, S, C, n_chains, n_steps);
 }
 
 template <int NUM, int TM>
 cudaError_t burgers_launch_team_forward(const BurgersDev &b, long long n, const double *u, double *G, double *phi,
                                        double *state, long long *work, cudaStream_t st) {
-    const size_t smem = burgers_team_smem_bytes(b.N);
-    auto kern = burgers_team_forward_kernel<32, NUM, TM>;
-    IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid_for(n), 32 * TM, smem, st>>>(b, n, u, G, phi, state, work);
-    IPMCMC_CU(cudaGetLastError());
-    return cudaSuccess;
+    return launch(burgers_team_forward_kernel<32, NUM, TM>, grid_for(n), 32 * TM, burgers_team_smem_bytes(b.N), st,
+                  b, n, u, G, phi, state, work);
 }
 template <int NUM, int TM>
 cudaError_t burgers_launch_team_chain(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,
                                      long long n_steps, cudaStream_t st) {
-    const size_t smem = burgers_team_smem_bytes(b.N);
-    auto kern = burgers_team_chain_kernel<32, NUM, TM>;
-    IPMCMC_CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid_for(n_chains), 32 * TM, smem, st>>>(b, S, C, n_chains, n_steps);
-    IPMCMC_CU(cudaGetLastError());
-    return cudaSuccess;
+    return launch(burgers_team_chain_kernel<32, NUM, TM>, grid_for(n_chains), 32 * TM, burgers_team_smem_bytes(b.N), st,
+                  b, S, C, n_chains, n_steps);
 }
 
 }  // namespace ipmcmc

@@ -13,6 +13,31 @@ constexpr unsigned FULL = 0xffffffffu;
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 
+// Developer instrumentation (-DIPMCMC_PROF=1, tools/overhead_probe.py): cycles per section of a work
+// item, summed over all warps by lane 0.  Not compiled into the product library.
+#ifndef IPMCMC_PROF
+#define IPMCMC_PROF 0
+#endif
+#if IPMCMC_PROF
+static __device__ unsigned long long g_prof[16];
+#define PROF_T(var) const long long var = clock64()
+#define PROF_ADD(slot, a, b) do { if (lane_id() == 0) atomicAdd(&g_prof[slot], (unsigned long long)((b) - (a))); } while (0)
+#else
+#define PROF_T(var)
+#define PROF_ADD(slot, a, b)
+#endif
+
+// grid.x for n_blocks CTAs (clamped to the largest grid.x; the kernels stride over the rest)
+inline int grid_for(long long n_blocks) { return (int)(n_blocks < 2147483647LL ? n_blocks : 2147483647LL); }
+
+// number of SMs of the current device
+inline cudaError_t sm_count(int &n_sm) {
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+    return e;
+}
+
 // 64-bit shuffles
 __device__ __forceinline__ double shfl(double v, int src, unsigned mask = FULL) { return __shfl_sync(mask, v, src); }
 __device__ __forceinline__ double shfl_up1(double v) { return __shfl_up_sync(FULL, v, 1); }

@@ -219,8 +219,6 @@ extern "C" int ipmcmc_lorenz_create(const ipmcmc_lorenz_desc *d, ipmcmc_problem 
 // ------------------------------------------------------------------------------------------------
 // dispatch
 // ------------------------------------------------------------------------------------------------
-static int grid_for(long long n_blocks) { return (int)(n_blocks < 2147483647LL ? n_blocks : 2147483647LL); }
-
 static int cu(cudaError_t e) {
     if (e != cudaSuccess) return fail(IPMCMC_ECUDA, "kernel launch: %s", cudaGetErrorString(e));
     return 0;
@@ -259,13 +257,11 @@ static int cu(cudaError_t e) {
 // warps per SM, so that the warps of an SM are dealt round-robin onto its four sub-partitions
 // (warp w -> sub-partition w % 4); larger batches use 4-warp CTAs and the block scheduler.
 static int lorenz_warps_per_cta(long long warps, int K) {
-    int dev = 0, n_sm = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+    int n_sm = 148;
+    sm_count(n_sm);
     int wpc = warps <= 8LL * n_sm ? (int)((warps + n_sm - 1) / n_sm) : 4;
     if (const char *e = getenv("IPMCMC_LORENZ_WPC")) wpc = atoi(e) > 0 && atoi(e) <= 8 ? atoi(e) : wpc;  // experiments
-    const int fit = (int)((48 * 1024) / lorenz_smem_bytes(K));   // default dynamic shared memory limit
-    if (wpc > fit) wpc = fit;
+    if (wpc > lorenz_warps_fit(K)) wpc = lorenz_warps_fit(K);
     return wpc < 1 ? 1 : wpc;
 }
 
@@ -419,7 +415,9 @@ extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const
     C.inject_u = b->inject_u_dev;
     C.slot_chain = b->slot_chain_dev;
     C.n_slots = b->n_slots;
-    C.sched = nullptr;
+    C.sched = (long long *)b->sched_dev;
+    int chunk = b->sched_chunk > 0 ? b->sched_chunk : 1;   // steps per work item of the dynamic scheduler
+    if (const char *e = getenv("IPMCMC_SCHED_CHUNK")) chunk = atoi(e) > 0 ? atoi(e) : chunk;  // experiments
     if (p->model == IPMCMC_MODEL_BURGERS) {
         int wpc = b->warps_per_cta > 0 ? b->warps_per_cta : 4;
         if (wpc > 8) return fail(IPMCMC_EINVAL, "warps_per_cta=%d > 8", wpc);
@@ -430,9 +428,6 @@ extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const
             if (b->sched_len < sched_len(n_chains))
                 return fail(IPMCMC_EINVAL, "sched_len=%lld < 3*n_chains+2", (long long)b->sched_len);
             if (n_chains >= (1LL << 31)) return fail(IPMCMC_EUNSUPPORTED, "dynamic scheduler: n_chains >= 2^31");
-            int chunk = b->sched_chunk > 0 ? b->sched_chunk : 1;
-            if (const char *e = getenv("IPMCMC_SCHED_CHUNK")) chunk = atoi(e) > 0 ? atoi(e) : chunk;  // experiments
-            C.sched = (long long *)b->sched_dev;
             BURGERS_DISPATCH(burgers_launch_chain_queue, p->b, S, C, n_chains, n_steps, chunk, st);
         }
         BURGERS_DISPATCH(burgers_launch_chain, p->b, S, C, n_chains, n_steps, wpc, st);
@@ -444,9 +439,8 @@ extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const
         // dynamic step scheduler over the warps' chain groups: persistent warps, one wave (255 registers:
         // 8 warps per SM at most; the queue needs every launched CTA resident)
         if (b->sched_len < sched_len(warps)) return fail(IPMCMC_EINVAL, "sched_len=%lld too short", (long long)b->sched_len);
-        int dev = 0, n_sm = 148;
-        CUDA_TRY(cudaGetDevice(&dev));
-        CUDA_TRY(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+        int n_sm = 148;
+        CUDA_TRY(sm_count(n_sm));
         long long ctas;
         int qwpc = wpc;
         if (warps <= 8LL * n_sm) {
@@ -454,18 +448,14 @@ extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const
             // chains: 80 SMs with 6 warps, 68 with 5, instead of 137 CTAs of 6 and 11 idle SMs)
             ctas = warps < n_sm ? warps : n_sm;
             qwpc = (int)((warps + ctas - 1) / ctas);
-            const int fit = (int)((48 * 1024) / lorenz_smem_bytes(p->l.K));
+            const int fit = lorenz_warps_fit(p->l.K);
             if (qwpc > fit) { qwpc = fit; ctas = (warps + qwpc - 1) / qwpc; }
         } else {
             const long long resident = (long long)n_sm * (8 / wpc);
             ctas = (warps + wpc - 1) / wpc;
             if (ctas > resident) ctas = resident;
         }
-        int chunk = b->sched_chunk > 0 ? b->sched_chunk : 1;
-        if (const char *e = getenv("IPMCMC_SCHED_CHUNK")) chunk = atoi(e) > 0 ? atoi(e) : chunk;  // experiments
-        C.sched = (long long *)b->sched_dev;
-        sched_init_kernel<<<(unsigned)((2 * warps + 255) / 256 < 1184 ? (2 * warps + 255) / 256 : 1184), 256, 0, st>>>(C.sched, warps);
-        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(sched_init(C.sched, warps, st));
         LORENZ_DISPATCH(lorenz_chain_queue_kernel, p->l.J, p->l.K, p->numerics,
                         <<<(int)ctas, 32 * qwpc, qwpc * lorenz_smem_bytes(p->l.K), st>>>(p->l, S, C, n_chains, n_steps, chunk));
         return 0;
@@ -842,9 +832,8 @@ __global__ void __launch_bounds__(256) dfma_peak_kernel(double *out, int iters, 
 
 extern "C" int ipmcmc_fp64_peak(int32_t iters, double *tflops_out) {
     if (!tflops_out) return fail(IPMCMC_EINVAL, "NULL argument");
-    int dev = 0, sms = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    CUDA_TRY(sm_count(sms));
     double *out;
     CUDA_TRY(cudaMalloc((void **)&out, 8));
     const int inner = 2048, blocks = sms * 8;

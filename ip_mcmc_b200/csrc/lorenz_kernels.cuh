@@ -12,6 +12,8 @@ __host__ __device__ inline int lorenz_groups(int K) { return 32 / K; }
 __host__ __device__ inline size_t lorenz_smem_bytes(int K) {
     return (size_t)(lorenz_groups(K) + 1) * 2 * IPMCMC_MAX_OBS * sizeof(double);
 }
+// warps per CTA whose shared memory fits the default dynamic shared-memory limit of 48 KB
+inline int lorenz_warps_fit(int K) { return (int)((48 * 1024) / lorenz_smem_bytes(K)); }
 
 template <int J, int KT, int NUM>
 __device__ __forceinline__ void lorenz_load_state(const LorenzLanes<J, KT, NUM> &L, const double *s, double (&y)[J + 1]) {
@@ -97,18 +99,8 @@ __global__ void __launch_bounds__(256, 1) lorenz_forward_kernel(const __grid_con
     }
 }
 
-// Global loads/stores of the chain state.  Under the dynamic scheduler (QUEUE) another SM may have
-// written the state earlier in the same launch: go through L2 (L1 is not coherent).
-template <bool QUEUE, class T>
-__device__ __forceinline__ T ld_state(const T *p) { return QUEUE ? __ldcg(p) : *p; }
-template <bool QUEUE, class T>
-__device__ __forceinline__ void st_state(T *p, T v) {
-    if (QUEUE) __stcg(p, v);
-    else *p = v;
-}
-
 // Metropolis steps [s0, s1) of the launch for the warp's group of chains c0 .. c0 + groups - 1
-// (chain c0 + slot on this lane group): load the chain state, step, store it back.
+// (chain c0 + slot on this lane group): load the chain state (ld_state<QUEUE>, sched.cuh), step, store it back.
 template <int J, int KT, int NUM, bool QUEUE>
 __device__ __forceinline__ void lorenz_advance_group(const LorenzDev &P, const SamplerDev &Sd, const ChainBufDev &C,
                                                      const LorenzLanes<J, KT, NUM> &L, const Group &Gp, int slot,
@@ -271,36 +263,9 @@ __global__ void __launch_bounds__(256, 1) lorenz_chain_queue_kernel(const __grid
     // the launch spreads ceil(n_units / n_CTA) warps per CTA over ALL SMs (engine.cu); the surplus warps of
     // the last rows leave at once instead of spinning on an empty queue beside a working warp
     if ((long long)warp * gridDim.x + blockIdx.x >= n_units) return;
-    SchedView Q(C.sched, n_units);
-    const unsigned long long cap = (unsigned long long)Q.cap;
-    const long long items_per_unit = (n_steps + chunk - 1) / chunk;
-    const unsigned long long total = (unsigned long long)n_units * (unsigned long long)items_per_unit;
-    while (true) {
-        unsigned long long idx = 0;
-        if (lane == 0) idx = atomicAdd(Q.head, 1ull);
-        idx = __shfl_sync(FULL, idx, 0);
-        if (idx >= total) break;
-        unsigned long long *rslot = Q.ring + idx % cap;
-        const unsigned long long want = idx / cap + 1;
-        const unsigned long long e = spin_until(rslot, lane, [want](unsigned long long v) { return (v >> 32) == want; });
-        if (lane == 0) st_relaxed_u64(rslot, 0ull);
-        __syncwarp();
-        const long long g = (long long)(e & 0xffffffffull);
-        const long long s0 = __ldcg(Q.progress + g);
-        const long long s1 = (s0 + chunk < n_steps) ? s0 + chunk : n_steps;
+    sched_serve(C.sched, n_units, n_steps, chunk, lane, [&](long long g, long long s0, long long s1) {
         lorenz_advance_group<J, KT, NUM, true>(P, Sd, C, L, Gp, slot, Gs, r2, n_chains, n_steps, g * groups, s0, s1);
-        if (lane == 0) __stcg(Q.progress + g, s1);
-        __syncwarp();
-        if (s1 < n_steps) {   // warp-uniform
-            unsigned long long t = 0;
-            if (lane == 0) t = atomicAdd(Q.tail, 1ull);
-            t = __shfl_sync(FULL, t, 0);
-            unsigned long long *pslot = Q.ring + t % cap;
-            spin_until(pslot, lane, [](unsigned long long v) { return v == 0ull; });
-            if (lane == 0) st_release_u64(pslot, ((t / cap + 1) << 32) | (unsigned long long)g);
-        }
-        __syncwarp();
-    }
+    });
 }
 
 // ---- probes -------------------------------------------------------------------------------

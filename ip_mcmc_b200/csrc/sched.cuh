@@ -53,6 +53,13 @@ static __global__ void sched_init_kernel(long long *sched, long long n_chains) {
     }
 }
 
+// Queues work units 0 .. n_units - 1, each at step 0, on stream st (ahead of the kernel that serves them).
+static inline cudaError_t sched_init(long long *sched, long long n_units, cudaStream_t st) {
+    const long long blocks = (2 * n_units + 255) / 256;
+    sched_init_kernel<<<(unsigned)(blocks < 1184 ? blocks : 1184), 256, 0, st>>>(sched, n_units);
+    return cudaGetLastError();
+}
+
 // Spin until lane 0 reads a value accepted by `ok` from *p; returns it on every lane.  The loop
 // condition is warp-uniform (lane 0 only issues a predicated load): a lane spinning on its own
 // does not reconverge with the other 31, and the whole solve would then run twice, once per part
@@ -68,5 +75,67 @@ __device__ __forceinline__ unsigned long long spin_until(const unsigned long lon
     }
 }
 
+// Global loads/stores of the chain state.  Under the dynamic scheduler (QUEUE) another SM may have
+// written the state earlier in the same launch: go through L2 (L1 is not coherent).
+template <bool QUEUE, class T>
+__device__ __forceinline__ T ld_state(const T *p) { return QUEUE ? __ldcg(p) : *p; }
+template <bool QUEUE, class T>
+__device__ __forceinline__ void st_state(T *p, T v) {
+    if (QUEUE) __stcg(p, v);
+    else *p = v;
+}
+
+// The warp's serving loop, called by all 32 lanes: take a ticket, wait for its ring slot, consume it,
+// run `body(unit, s0, s1)` (steps [s0, s1) of the launch for that work unit, `chunk` at most), and push
+// the unit back while it has steps left; returns when every item has been taken.
+// The unit's state -- what `body` stored with st_state<true>, its counters and its progress -- is
+// published to the next warp by the release store of the ring entry (no separate fence): the other
+// lanes' stores are ordered before it by __syncwarp (cumulativity), and the next warp's acquire load
+// of the entry, followed by __syncwarp, orders all its lanes' loads after it.  A unit sits in the ring
+// at most once, so one warp at a time owns it and read-modify-writes of its state need no atomics.
+template <class Body>
+__device__ __forceinline__ void sched_serve(long long *sched, long long n_units, long long n_steps, int chunk, int lane,
+                                            const Body &body) {
+    const SchedView Q(sched, n_units);
+    const unsigned long long cap = (unsigned long long)Q.cap;
+    const long long items_per_unit = (n_steps + chunk - 1) / chunk;
+    const unsigned long long total = (unsigned long long)n_units * (unsigned long long)items_per_unit;
+    while (true) {
+        PROF_T(t0);
+        unsigned long long idx = 0;
+        if (lane == 0) idx = atomicAdd(Q.head, 1ull);
+        idx = __shfl_sync(FULL, idx, 0);
+        if (idx >= total) break;
+        unsigned long long *slot = Q.ring + idx % cap;
+        const unsigned long long want = idx / cap + 1;
+        const unsigned long long e = spin_until(slot, lane, [want](unsigned long long v) { return (v >> 32) == want; });
+        // mark the slot consumed: ordered after our own read of it (same address), nothing to publish
+        if (lane == 0) st_relaxed_u64(slot, 0ull);
+        __syncwarp();
+        const long long unit = (long long)(e & 0xffffffffull);
+        const long long s0 = __ldcg(Q.progress + unit);
+        const long long s1 = (s0 + chunk < n_steps) ? s0 + chunk : n_steps;
+        PROF_T(t1);
+        body(unit, s0, s1);
+        PROF_T(t2);
+        if (lane == 0) __stcg(Q.progress + unit, s1);
+        __syncwarp();
+        if (s1 < n_steps) {   // warp-uniform
+            unsigned long long t = 0;
+            if (lane == 0) t = atomicAdd(Q.tail, 1ull);
+            t = __shfl_sync(FULL, t, 0);
+            unsigned long long *pslot = Q.ring + t % cap;
+            spin_until(pslot, lane, [](unsigned long long v) { return v == 0ull; });   // previous lap consumed (cap = 2n: no wait in practice)
+            if (lane == 0) st_release_u64(pslot, ((t / cap + 1) << 32) | (unsigned long long)unit);
+        }
+        __syncwarp();
+        PROF_T(t3);
+        PROF_ADD(0, t0, t3);
+        PROF_ADD(1, t0, t1);
+        PROF_ADD(6, t1, t2);
+        PROF_ADD(7, t2, t3);
+        PROF_ADD(8, 0, 1);
+    }
+}
 
 }  // namespace ipmcmc

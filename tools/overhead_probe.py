@@ -62,8 +62,8 @@ if lib is not None and hasattr(lib, "ipmcmc_prof_read"):
         v = np.array(list(buf), dtype=np.float64)
         items = v[8]
         nfv = (ch.counters[:, 2].sum().item() - c0) / items
-        names = ["item total", "pop (ticket, ring, state loads)", "proposal noise", "integrate (IC + time loop)",
-                 "store + measure + Phi", "accept (exp, U, update)", "all Metropolis steps", "write-back + push"]
+        names = ["item total", "pop (ticket, ring, progress)", "proposal noise", "integrate (IC + time loop)",
+                 "store + measure + Phi", "accept (exp, U, update)", "state load + steps + write-back", "push"]
         print("chains=%d: %d items, %.1f FV steps per item" % (nch, items, nfv))
         for k, nm in enumerate(names):
             print("   %-34s %9.0f cycles per item  (%5.1f %%)" % (nm, v[k] / items, 100 * v[k] / v[0]))
