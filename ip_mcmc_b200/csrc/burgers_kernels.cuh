@@ -38,8 +38,32 @@ __device__ __forceinline__ void burgers_measure(const BurgersDev &B, const doubl
     __syncwarp();
 }
 
+// G and Phi of the absolute parameters `param`, given as BurgersWarp::integrate takes them: parameter i on
+// lane i (d <= 32) or a ParamAt functor (d > 32).  Leaves the end state in smem `state` and G in `Gs`.
+// Returns Phi; n_fv by reference.
+template <int CPL, int NUMERICS, bool PADDED, class Param>
+__device__ __forceinline__ double burgers_solve_phi(const BurgersDev &B, const Param &param, double *state, double *Gs,
+                                                   double *r2, int lane, int &n_fv) {
+    BurgersWarp<CPL, NUMERICS, PADDED> W;
+    PROF_T(p0);
+    n_fv = W.integrate(B, param, lane);
+    PROF_T(p1);
+#pragma unroll
+    for (int k = 0; k < CPL; ++k) {
+        const int c = lane * CPL + k;
+        if (c < B.N) state[c] = W.u[k];
+    }
+    __syncwarp();
+    burgers_measure(B, state, Gs, lane);
+    const double phi = potential_from_G(B.pot, Gs, r2, lane, 32, FULL);
+    PROF_T(p2);
+    PROF_ADD(3, p0, p1);   // -DIPMCMC_PROF builds: every Burgers one-warp solve, the wide path's included
+    PROF_ADD(4, p1, p2);
+    // a solve stopped by the safety cap has not reached T: report it as non-finite (-> rejected)
+    return W.capped ? nan("") : phi;
+}
+
 // G(u) and Phi(u) for the parameter vector whose component i sits on lane i (value `ui`).
-// Leaves the end state in smem `state` and G in `Gs`.  Returns Phi; n_fv by reference.
 // Inlined at its call sites on purpose: with the solve as an out-of-line subroutine ptxas allocates the
 // time-step loop's registers around the call convention and schedules it measurably worse (B200,
 // 1024 x 256 cells: 60 % of the fp64 peak out of line, 66 % inlined; 8192 x 1024: 78 % / 83 %).
@@ -51,23 +75,7 @@ __device__ IPMCMC_PHI_INLINE double burgers_phi(const BurgersDev &B, double ui, 
                                               int lane, int &n_fv) {
     // FVMObservationOperator.__call__ (utilities.py:40-41): IC(u_0 + u)
     const double pi = (lane < B.d) ? B.param_mean[lane] + ui : 0.0;
-    BurgersWarp<CPL, NUMERICS, PADDED> W;
-    PROF_T(p0);
-    n_fv = W.integrate(B, pi, lane);
-    PROF_T(p1);
-#pragma unroll
-    for (int k = 0; k < CPL; ++k) {
-        const int c = lane * CPL + k;
-        if (c < B.N) state[c] = W.u[k];
-    }
-    __syncwarp();
-    burgers_measure(B, state, Gs, lane);
-    const double phi = potential_from_G(B.pot, Gs, r2, lane, 32, FULL);
-    PROF_T(p2);
-    PROF_ADD(3, p0, p1);
-    PROF_ADD(4, p1, p2);
-    // a solve stopped by the safety cap has not reached T: report it as non-finite (-> rejected)
-    return W.capped ? nan("") : phi;
+    return burgers_solve_phi<CPL, NUMERICS, PADDED>(B, pi, state, Gs, r2, lane, n_fv);
 }
 
 // Outputs of forward evaluation c (null pointers are skipped): G and the end state from shared memory,
@@ -107,59 +115,110 @@ __global__ void __launch_bounds__(256) burgers_forward_kernel(const __grid_const
     }
 }
 
-// Registers of one chain between Metropolis steps.
-struct ChainRegs {
-    double ui, phi_u, reg_u;
+// The chain's parameter vector u and its proposal v, component i on lane i (d <= 32): u and its Welford moments
+// in registers, v a register value; the free functions of sampler.cuh (shared with the Lorenz kernels) do the work.
+struct LaneVec {
+    double u;
     Welford mom;
+
+    // v = ca*u + cb*w (proposer.py:29-30, 81-82), logged to vlog
+    __device__ __forceinline__ double propose(const SamplerDev &S, const ChainBufDev &C, const Group &Gp, long long c,
+                                              long long cg, long long s, long long n_steps, long long gstep, double ca,
+                                              double cb, bool writer) const {
+        const double w = proposal_noise(S, C, Gp, c, cg, s, n_steps, gstep);
+        const double v = ca * u + cb * w;
+        if (writer && C.vlog && Gp.lane < S.d) C.vlog[(c * n_steps + s) * S.d + Gp.lane] = v;
+        return v;
+    }
+    __device__ __forceinline__ bool inside(const SamplerDev &S, const Group &Gp, double x) const {
+        return constraint_ok(S, Gp, x);
+    }
+    __device__ __forceinline__ double regulariser(const SamplerDev &S, const Group &Gp, double x) const {
+        return prior_regulariser(S, Gp, x);
+    }
+    __device__ __forceinline__ void accept(const SamplerDev &, const Group &, double v) { u = v; }
+    // recorded sample n_rec of the launch: moments, trace
+    __device__ __forceinline__ void record(const SamplerDev &S, const ChainBufDev &C, const Group &Gp, long long c,
+                                           long long n_rec, bool writer) {
+        mom.add(u);
+        if (writer && C.trace && n_rec < C.n_record && Gp.lane < S.d) C.trace[(c * C.n_record + n_rec) * S.d + Gp.lane] = u;
+    }
+    template <bool QUEUE>
+    __device__ __forceinline__ void load_u(const SamplerDev &S, const ChainBufDev &C, int lane, long long c) {
+        u = (lane < S.d) ? ld_state<QUEUE>(C.u + c * S.d + lane) : 0.0;
+    }
+    template <bool QUEUE>
+    __device__ __forceinline__ void load_moments(const SamplerDev &S, const ChainBufDev &C, int lane, long long c) {
+        const int d = S.d;
+        mom = Welford{ld_state<QUEUE>(C.mom_count + c), (lane < d) ? ld_state<QUEUE>(C.mom_mean + c * d + lane) : 0.0,
+                      (lane < d) ? ld_state<QUEUE>(C.mom_m2 + c * d + lane) : 0.0};
+    }
+    // u and the per-component moments; the count is stored by lane 0 (count())
+    template <bool QUEUE>
+    __device__ __forceinline__ void store(const SamplerDev &S, const ChainBufDev &C, int lane, long long c) const {
+        const int d = S.d;
+        if (lane < d) {
+            st_state<QUEUE>(C.u + c * d + lane, u);
+            st_state<QUEUE>(C.mom_mean + c * d + lane, mom.mean);
+            st_state<QUEUE>(C.mom_m2 + c * d + lane, mom.m2);
+        }
+    }
+    __device__ __forceinline__ double count() const { return mom.count; }
+};
+
+// Registers of one chain between Metropolis steps.  `Vec`: where its parameter vector lives, LaneVec or
+// SmemVec (wide path).
+template <class Vec>
+struct ChainRegs {
+    Vec x;
+    double phi_u, reg_u;
     long long cnt[CNT_N];
 };
 
 // ONE Metropolis step of chain c (local id; cg global id) at launch-local step s: proposal -> (box
 // constraint) -> solve -> Phi(v) -> accept/reject -> counters, logs, moments, trace.
-// `phi_of(ui, n_fv)` evaluates Phi for the parameter vector whose component i sits on lane i: the one-warp
-// solver (burgers_phi) or the multi-warp team solver (burgers_team_phi), whose warps all run this same step
-// with the same Philox draws; `writer` (warp 0 of a team; always true for one warp per chain) owns the
-// global-memory outputs.
+// `phi_of(x, n_fv)` evaluates Phi for a parameter vector of R's kind (R.x.u or the proposal): the one-warp
+// solver (burgers_phi), the multi-warp team solver (burgers_team_phi), whose warps all run this same step
+// with the same Philox draws, or the one-warp solver over a shared-memory vector (burgers_phi_wide); `writer`
+// (warp 0 of a team; always true for one warp per chain) owns the global-memory outputs.
 #ifndef IPMCMC_STEP_INLINE
 #define IPMCMC_STEP_INLINE __forceinline__
 #endif
-template <class PhiOf>
+template <class Vec, class PhiOf>
 __device__ IPMCMC_STEP_INLINE void metropolis_step(const SamplerDev &S, const ChainBufDev &C, const Group &Gp, long long c,
-                                                   long long cg, long long s, long long n_steps, ChainRegs &R,
+                                                   long long cg, long long s, long long n_steps, ChainRegs<Vec> &R,
                                                    const PhiOf &phi_of, bool writer) {
-    const int lane = Gp.lane, d = S.d;
+    const int lane = Gp.lane;
     const long long gstep = S.first_step + s;
     double ca, cb;
     PROF_T(q0);
     step_coefs(S, gstep, ca, cb);
-    const double w = proposal_noise(S, C, Gp, c, cg, s, n_steps, gstep);
-    const double vi = ca * R.ui + cb * w;
+    const auto v = R.x.propose(S, C, Gp, c, cg, s, n_steps, gstep, ca, cb, writer);
     PROF_T(q1);
     PROF_ADD(2, q0, q1);
-    if (writer && C.vlog && lane < d) C.vlog[(c * n_steps + s) * d + lane] = vi;
     bool accepted = false;
     double phi_v = nan(""), a = nan("");
     int n_fv = 0;
-    const bool ok = !S.has_constraint || constraint_ok(S, Gp, vi);
+    const bool ok = !S.has_constraint || R.x.inside(S, Gp, v);
     if (ok) {
         if (S.recompute_phi_u) {  // the reference's 2 solves per step (accepter.py:121-122)
             int nf0;
-            R.phi_u = phi_of(R.ui, nf0);
+            R.phi_u = phi_of(R.x.u, nf0);
             R.cnt[CNT_WORK_A] += nf0;
             R.cnt[CNT_WORK_B] += 1;
         }
-        phi_v = phi_of(vi, n_fv);
+        phi_v = phi_of(v, n_fv);
         PROF_T(q2);
         R.cnt[CNT_WORK_A] += n_fv;
         R.cnt[CNT_WORK_B] += 1;
         double reg_v = 0.0;
-        if (S.accepter == IPMCMC_ACCEPT_RW) reg_v = prior_regulariser(S, Gp, vi);
+        if (S.accepter == IPMCMC_ACCEPT_RW) reg_v = R.x.regulariser(S, Gp, v);
         a = exp((R.phi_u + R.reg_u) - (phi_v + reg_v));
         const double U = C.inject_u ? C.inject_u[c * n_steps + s] : draw_uniform(S.seed, (uint64_t)cg, (uint64_t)gstep);
         accepted = a > U;  // strict, un-clipped; NaN compares false (accepter.py:61-62)
         if (!isfinite(phi_v)) R.cnt[CNT_NONFINITE] += 1;
         if (accepted) {
-            R.ui = vi;
+            R.x.accept(S, Gp, v);
             R.phi_u = phi_v;
             R.reg_u = reg_v;
         }
@@ -178,52 +237,42 @@ __device__ IPMCMC_STEP_INLINE void metropolis_step(const SamplerDev &S, const Ch
         L[3] = (double)n_fv;
     }
     // recording (sampler.py:23-28)
-    if (records_step(S, gstep)) {
-        R.mom.add(R.ui);
-        const long long n_rec = recorded_before(S, gstep) - recorded_before(S, S.first_step);
-        if (writer && C.trace && n_rec < C.n_record && lane < d) C.trace[(c * C.n_record + n_rec) * d + lane] = R.ui;
-    }
+    if (records_step(S, gstep)) R.x.record(S, C, Gp, c, recorded_before(S, gstep) - recorded_before(S, S.first_step), writer);
 }
 
-// Chain c's registers from global memory (ld_state<QUEUE>).  On the chain's first launch Phi(u_0) is not
-// known yet (NaN) and is solved for with `phi_of`.  `team`: every warp of the CTA runs this for the same
-// chain, and all must have read the state before warp 0 may overwrite it (burgers_store_chain).
-template <bool QUEUE, class PhiOf>
-__device__ __forceinline__ ChainRegs burgers_load_chain(const SamplerDev &S, const ChainBufDev &C, const Group &Gp,
-                                                        long long c, const PhiOf &phi_of, bool team) {
-    const int lane = Gp.lane, d = S.d;
-    ChainRegs R;
-    R.ui = (lane < d) ? ld_state<QUEUE>(C.u + c * d + lane) : 0.0;
+// Chain c's registers from global memory (ld_state<QUEUE>); `x` says where the parameter vector goes.  On the
+// chain's first launch Phi(u_0) is not known yet (NaN) and is solved for with `phi_of`.  `team`: every warp of
+// the CTA runs this for the same chain, and all must have read the state before warp 0 may overwrite it
+// (burgers_store_chain).
+template <bool QUEUE, class Vec, class PhiOf>
+__device__ __forceinline__ ChainRegs<Vec> burgers_load_chain(const SamplerDev &S, const ChainBufDev &C, const Group &Gp,
+                                                             long long c, const Vec &x, const PhiOf &phi_of, bool team) {
+    ChainRegs<Vec> R{x};
+    R.x.template load_u<QUEUE>(S, C, Gp.lane, c);
     R.phi_u = ld_state<QUEUE>(C.phi + c);
 #pragma unroll
     for (int k = 0; k < CNT_N; ++k) R.cnt[k] = 0;
     if (team) __syncthreads();
     if (isnan(R.phi_u)) {
         int n_fv;
-        R.phi_u = phi_of(R.ui, n_fv);
+        R.phi_u = phi_of(R.x.u, n_fv);
         R.cnt[CNT_WORK_A] += n_fv;
         R.cnt[CNT_WORK_B] += 1;
     }
-    R.reg_u = (S.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser(S, Gp, R.ui) : 0.0;
-    R.mom = Welford{ld_state<QUEUE>(C.mom_count + c), (lane < d) ? ld_state<QUEUE>(C.mom_mean + c * d + lane) : 0.0,
-                    (lane < d) ? ld_state<QUEUE>(C.mom_m2 + c * d + lane) : 0.0};
+    R.reg_u = (S.accepter == IPMCMC_ACCEPT_RW) ? R.x.regulariser(S, Gp, R.x.u) : 0.0;
+    R.x.template load_moments<QUEUE>(S, C, Gp.lane, c);
     return R;
 }
 
 // Chain c's registers back to global memory; the counters accumulate over launches.  A chain belongs to
 // one warp (or team) at a time, so their read-modify-write needs no atomic, under the queue too (sched.cuh).
-template <bool QUEUE>
+template <bool QUEUE, class Vec>
 __device__ __forceinline__ void burgers_store_chain(const SamplerDev &S, const ChainBufDev &C, int lane, long long c,
-                                                    const ChainRegs &R) {
-    const int d = S.d;
-    if (lane < d) {
-        st_state<QUEUE>(C.u + c * d + lane, R.ui);
-        st_state<QUEUE>(C.mom_mean + c * d + lane, R.mom.mean);
-        st_state<QUEUE>(C.mom_m2 + c * d + lane, R.mom.m2);
-    }
+                                                    const ChainRegs<Vec> &R) {
+    R.x.template store<QUEUE>(S, C, lane, c);
     if (lane == 0) {
         st_state<QUEUE>(C.phi + c, R.phi_u);
-        st_state<QUEUE>(C.mom_count + c, R.mom.count);
+        st_state<QUEUE>(C.mom_count + c, R.x.count());
 #pragma unroll
         for (int k = 0; k < CNT_N; ++k)
             st_state<QUEUE>(C.counters + c * CNT_N + k, ld_state<QUEUE>(C.counters + c * CNT_N + k) + R.cnt[k]);
@@ -242,17 +291,15 @@ struct BurgersPhiOf {
     }
 };
 
-// Metropolis steps [s0, s1) of the launch for chain c on one warp: load the chain state, step, store it back.
-template <int CPL, int NUMERICS, bool PADDED, bool QUEUE>
-__device__ __forceinline__ void burgers_advance_chain(const BurgersDev &B, const SamplerDev &S, const ChainBufDev &C,
-                                                      const Group &Gp, long long c, long long s0, long long s1,
-                                                      long long n_steps, double *state, double *Gs, double *r2) {
-    const int lane = Gp.lane;
+// Metropolis steps [s0, s1) of the launch for chain c on one warp: load the chain state into `x`, step, store it back.
+template <bool QUEUE, class Vec, class PhiOf>
+__device__ __forceinline__ void burgers_advance_chain(const SamplerDev &S, const ChainBufDev &C, const Group &Gp,
+                                                      long long c, long long s0, long long s1, long long n_steps,
+                                                      const Vec &x, const PhiOf &phi_of) {
     const long long cg = S.chain_offset + c;
-    const BurgersPhiOf<CPL, NUMERICS, PADDED> phi_of{B, state, Gs, r2, lane};
-    ChainRegs R = burgers_load_chain<QUEUE>(S, C, Gp, c, phi_of, false);
+    ChainRegs<Vec> R = burgers_load_chain<QUEUE>(S, C, Gp, c, x, phi_of, false);
     for (long long s = s0; s < s1; ++s) metropolis_step(S, C, Gp, c, cg, s, n_steps, R, phi_of, true);
-    burgers_store_chain<QUEUE>(S, C, lane, c, R);
+    burgers_store_chain<QUEUE>(S, C, Gp.lane, c, R);
     __syncwarp();
 }
 
@@ -272,7 +319,8 @@ __global__ void __launch_bounds__(256, IPMCMC_CHAIN_MINB(CPL)) burgers_chain_ker
     for (long long slot = (long long)blockIdx.x * wpc + warp; slot < n_slots; slot += (long long)gridDim.x * wpc) {
         const long long c = C.slot_chain ? (long long)C.slot_chain[slot] : slot;
         if (c < 0 || c >= n_chains) continue;
-        burgers_advance_chain<CPL, NUMERICS, PADDED, false>(B, S, C, Gp, c, 0, n_steps, n_steps, state, Gs, r2);
+        burgers_advance_chain<false>(S, C, Gp, c, 0, n_steps, n_steps, LaneVec{},
+                                     BurgersPhiOf<CPL, NUMERICS, PADDED>{B, state, Gs, r2, Gp.lane});
     }
 }
 
@@ -290,7 +338,8 @@ __global__ void __launch_bounds__(256, MINB) burgers_chain_queue_kernel(
     const int lane = lane_id();
     const Group Gp{0, 32, lane, FULL};
     sched_serve(C.sched, n_chains, n_steps, chunk, lane, [&](long long c, long long s0, long long s1) {
-        burgers_advance_chain<CPL, NUMERICS, PADDED, true>(B, S, C, Gp, c, s0, s1, n_steps, state, Gs, r2);
+        burgers_advance_chain<true>(S, C, Gp, c, s0, s1, n_steps, LaneVec{},
+                                    BurgersPhiOf<CPL, NUMERICS, PADDED>{B, state, Gs, r2, lane});
     });
 }
 
@@ -299,9 +348,10 @@ __global__ void __launch_bounds__(256, MINB) burgers_chain_queue_kernel(
 // with up to 253 modes.  One chain per warp as before, but the parameter vector no longer fits the lanes
 // of the warp: u, the proposal v and the absolute parameters live in shared memory (component i is served
 // by lane i % 32), the solver reads its parameters from there (BurgersWarp::integrate over a ParamAt
-// functor), the running moments are updated in place in global memory.  Same Philox draws (slot = component),
-// same accept rule; diagonal sampling factor and diagonal prior factor only (what a KL prior is); static
-// chain -> warp map.  CPU statement: oracle/mcmc_np.run_chain + oracle/burgers_np with kl_basis.
+// functor).  The chain runs the same metropolis_step, burgers_load_chain and burgers_store_chain as the
+// one-warp kernels, over SmemVec instead of LaneVec: same Philox draws (slot = component), same accept rule;
+// diagonal sampling factor and diagonal prior factor only (what a KL prior is); static chain -> warp map.
+// CPU statement: oracle/mcmc_np.run_chain + oracle/burgers_np with kl_basis.
 // ------------------------------------------------------------------------------------------------
 // shared memory per warp: state[N] | G[MAX_OBS] | r2[MAX_OBS] | par[d] | u[d] | v[d]
 __host__ __device__ inline size_t burgers_wide_smem_bytes(int N, int d, int warps = 1) {
@@ -314,18 +364,20 @@ __device__ __forceinline__ double burgers_phi_wide(const BurgersDev &B, const do
                                                    double *Gs, double *r2, int lane, int &n_fv) {
     for (int i = lane; i < B.d; i += 32) par[i] = B.param_mean_wide[i] + x[i];   // utilities.py:41
     __syncwarp();
-    BurgersWarp<CPL, NUMERICS, PADDED> W;
-    n_fv = W.integrate(B, [par](int i) { return par[i]; }, lane);
-#pragma unroll
-    for (int k = 0; k < CPL; ++k) {
-        const int c = lane * CPL + k;
-        if (c < B.N) state[c] = W.u[k];
-    }
-    __syncwarp();
-    burgers_measure(B, state, Gs, lane);
-    const double phi = potential_from_G(B.pot, Gs, r2, lane, 32, FULL);
-    return W.capped ? nan("") : phi;
+    return burgers_solve_phi<CPL, NUMERICS, PADDED>(B, [par](int i) { return par[i]; }, state, Gs, r2, lane, n_fv);
 }
+
+// `phi_of` of the one-warp solver over a shared-memory parameter vector; a functor for the reason given at
+// BurgersPhiOf.
+template <int CPL, int NUMERICS, bool PADDED>
+struct BurgersWidePhiOf {
+    const BurgersDev &B;
+    double *par, *state, *Gs, *r2;
+    int lane;
+    __device__ __forceinline__ double operator()(const double *x, int &n_fv) const {
+        return burgers_phi_wide<CPL, NUMERICS, PADDED>(B, x, par, state, Gs, r2, lane, n_fv);
+    }
+};
 
 // sum over the warp in a fixed order (lane tree), the same bits on every lane
 __device__ __forceinline__ double warp_sum_fixed(double v) {
@@ -337,16 +389,92 @@ __device__ __forceinline__ double warp_sum_fixed(double v) {
     return v;
 }
 
-// 0.5 * ||L x||^2 for a diagonal L (accepter.py:104-106)
-__device__ __forceinline__ double prior_regulariser_wide(const SamplerDev &S, const double *x, int lane) {
-    double ss = 0.0;
-    for (int i = lane; i < S.d; i += 32) {
-        const double y = S.prior_chol_diag[i] * x[i];
-        ss = ss + y * y;
+// The chain's parameter vector u and its proposal v in shared memory, component i on lane i % 32 (d > 32).
+// The Welford moments are updated in place in global memory, their count is kept in a register.
+struct SmemVec {
+    double *u, *v;   // [d] each, in the warp's shared memory
+    double n;        // Welford count
+
+    // v = ca*u + cb*w (proposer.py:29-30, 81-82), w_i = factor_i * z_i, z_i = Philox slot i; logged to vlog
+    __device__ __forceinline__ const double *propose(const SamplerDev &S, const ChainBufDev &C, const Group &Gp,
+                                                     long long c, long long cg, long long s, long long n_steps,
+                                                     long long gstep, double ca, double cb, bool writer) const {
+        const int d = S.d;
+        for (int i = Gp.lane; i < d; i += 32) {
+            double w;
+            if (C.inject_w) {
+                w = C.inject_w[(c * n_steps + s) * d + i];
+            } else {
+                const double z = draw_normal(S.seed, (uint64_t)cg, (uint64_t)gstep, (uint32_t)i);
+                w = S.factor_kind == 1 ? S.factor[i] * z : z;
+            }
+            const double vi = ca * u[i] + cb * w;
+            v[i] = vi;
+            if (writer && C.vlog) C.vlog[(c * n_steps + s) * d + i] = vi;
+        }
+        __syncwarp();
+        return v;
     }
-    const double nrm = sqrt(warp_sum_fixed(ss));
-    return 0.5 * (nrm * nrm);
-}
+    // the box lo | hi | shift from the device table S.box_wide; all lanes agree
+    __device__ __forceinline__ bool inside(const SamplerDev &S, const Group &Gp, const double *x) const {
+        const int d = S.d;
+        bool in = true;
+        for (int i = Gp.lane; i < d; i += 32) {
+            const double sh = x[i] + S.box_wide[2 * d + i];
+            in = in && (sh > S.box_wide[i]) && (sh < S.box_wide[d + i]);
+        }
+        return __all_sync(FULL, in);
+    }
+    // 0.5 * ||L x||^2 for a diagonal L (accepter.py:104-106)
+    __device__ __forceinline__ double regulariser(const SamplerDev &S, const Group &Gp, const double *x) const {
+        const int d = S.d;
+        double ss = 0.0;
+        for (int i = Gp.lane; i < d; i += 32) {
+            const double y = S.prior_chol_diag[i] * x[i];
+            ss = ss + y * y;
+        }
+        const double nrm = sqrt(warp_sum_fixed(ss));
+        return 0.5 * (nrm * nrm);
+    }
+    __device__ __forceinline__ void accept(const SamplerDev &S, const Group &Gp, const double *x) {
+        const int d = S.d;
+        for (int i = Gp.lane; i < d; i += 32) u[i] = x[i];
+        __syncwarp();
+    }
+    // recorded sample n_rec of the launch: Welford in place, trace
+    __device__ __forceinline__ void record(const SamplerDev &S, const ChainBufDev &C, const Group &Gp, long long c,
+                                           long long n_rec, bool writer) {
+        const int d = S.d;
+        n += 1.0;
+        for (int i = Gp.lane; i < d; i += 32) {
+            const double x = u[i], m0 = C.mom_mean[c * d + i];
+            const double delta = x - m0, m1 = m0 + delta / n;
+            C.mom_mean[c * d + i] = m1;
+            C.mom_m2[c * d + i] += delta * (x - m1);
+            if (writer && C.trace && n_rec < C.n_record) C.trace[(c * C.n_record + n_rec) * d + i] = x;
+        }
+    }
+    template <bool QUEUE>
+    __device__ __forceinline__ void load_u(const SamplerDev &S, const ChainBufDev &C, int lane, long long c) {
+        const int d = S.d;
+        // unrolled by 4 as the compiler unrolled these copies when they were written out in the kernel: fewer
+        // spills in the wide kernels (ptxas -v)
+#pragma unroll 4
+        for (int i = lane; i < d; i += 32) u[i] = ld_state<QUEUE>(C.u + c * d + i);
+        __syncwarp();
+    }
+    template <bool QUEUE>
+    __device__ __forceinline__ void load_moments(const SamplerDev &, const ChainBufDev &C, int, long long c) {
+        n = ld_state<QUEUE>(C.mom_count + c);
+    }
+    template <bool QUEUE>
+    __device__ __forceinline__ void store(const SamplerDev &S, const ChainBufDev &C, int lane, long long c) const {
+        const int d = S.d;
+#pragma unroll 4
+        for (int i = lane; i < d; i += 32) st_state<QUEUE>(C.u + c * d + i, u[i]);
+    }
+    __device__ __forceinline__ double count() const { return n; }
+};
 
 template <int CPL, int NUMERICS, bool PADDED>
 __global__ void __launch_bounds__(128) burgers_wide_forward_kernel(const __grid_constant__ BurgersDev B, long long n,
@@ -377,104 +505,10 @@ __global__ void __launch_bounds__(128) burgers_wide_chain_kernel(const __grid_co
     const int warp = threadIdx.x >> 5, wpc = blockDim.x >> 5, d = S.d;
     double *smem = smem_all + (size_t)warp * (B.N + 2 * IPMCMC_MAX_OBS + 3 * d);
     double *state = smem, *Gs = smem + B.N, *r2 = Gs + IPMCMC_MAX_OBS, *par = r2 + IPMCMC_MAX_OBS, *us = par + d, *vs = us + d;
-    const int lane = lane_id();
-    for (long long c = (long long)blockIdx.x * wpc + warp; c < n_chains; c += (long long)gridDim.x * wpc) {
-        const long long cg = S.chain_offset + c;
-        for (int i = lane; i < d; i += 32) us[i] = C.u[c * d + i];
-        __syncwarp();
-        double phi_u = C.phi[c];
-        long long cnt[CNT_N];
-#pragma unroll
-        for (int k = 0; k < CNT_N; ++k) cnt[k] = 0;
-        if (isnan(phi_u)) {  // first launch: Phi(u_0) not known yet
-            int n_fv;
-            phi_u = burgers_phi_wide<CPL, NUMERICS, PADDED>(B, us, par, state, Gs, r2, lane, n_fv);
-            cnt[CNT_WORK_A] += n_fv;
-            cnt[CNT_WORK_B] += 1;
-        }
-        double reg_u = (S.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser_wide(S, us, lane) : 0.0;
-        double count = C.mom_count[c];
-        for (long long s = 0; s < n_steps; ++s) {
-            const long long gstep = S.first_step + s;
-            double ca, cb;
-            step_coefs(S, gstep, ca, cb);
-            // proposal (proposer.py:29-30, 81-82): v = ca*u + cb*w, w_i = factor_i * z_i, z_i = Philox slot i
-            bool inside = true;
-            for (int i = lane; i < d; i += 32) {
-                double w;
-                if (C.inject_w) {
-                    w = C.inject_w[(c * n_steps + s) * d + i];
-                } else {
-                    const double z = draw_normal(S.seed, (uint64_t)cg, (uint64_t)gstep, (uint32_t)i);
-                    w = S.factor_kind == 1 ? S.factor[i] * z : z;
-                }
-                const double vi = ca * us[i] + cb * w;
-                vs[i] = vi;
-                if (C.vlog) C.vlog[(c * n_steps + s) * d + i] = vi;
-                if (S.has_constraint) {
-                    const double sh = vi + S.box_wide[2 * d + i];
-                    inside = inside && (sh > S.box_wide[i]) && (sh < S.box_wide[d + i]);
-                }
-            }
-            __syncwarp();
-            const bool ok = !S.has_constraint || __all_sync(FULL, inside);
-            bool accepted = false;
-            double phi_v = nan(""), a = nan("");
-            int n_fv = 0;
-            if (ok) {
-                if (S.recompute_phi_u) {  // the reference's 2 solves per step (accepter.py:121-122)
-                    int nf0;
-                    phi_u = burgers_phi_wide<CPL, NUMERICS, PADDED>(B, us, par, state, Gs, r2, lane, nf0);
-                    cnt[CNT_WORK_A] += nf0;
-                    cnt[CNT_WORK_B] += 1;
-                }
-                phi_v = burgers_phi_wide<CPL, NUMERICS, PADDED>(B, vs, par, state, Gs, r2, lane, n_fv);
-                cnt[CNT_WORK_A] += n_fv;
-                cnt[CNT_WORK_B] += 1;
-                const double reg_v = (S.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser_wide(S, vs, lane) : 0.0;
-                a = exp((phi_u + reg_u) - (phi_v + reg_v));
-                const double U = C.inject_u ? C.inject_u[c * n_steps + s] : draw_uniform(S.seed, (uint64_t)cg, (uint64_t)gstep);
-                accepted = a > U;  // strict, un-clipped; NaN compares false (accepter.py:61-62)
-                if (!isfinite(phi_v)) cnt[CNT_NONFINITE] += 1;
-                if (accepted) {
-                    for (int i = lane; i < d; i += 32) us[i] = vs[i];
-                    phi_u = phi_v;
-                    reg_u = reg_v;
-                }
-                __syncwarp();
-            } else {
-                cnt[CNT_CONSTRAINT] += 1;
-            }
-            cnt[CNT_CALLS] += 1;
-            cnt[CNT_ACCEPTS] += accepted ? 1 : 0;
-            if (C.steplog && lane == 0) {
-                double *L = C.steplog + (c * n_steps + s) * 4;
-                L[0] = phi_v;
-                L[1] = a;
-                L[2] = accepted ? 1.0 : 0.0;
-                L[3] = (double)n_fv;
-            }
-            if (records_step(S, gstep)) {   // Welford in place (sampler.py:23-28)
-                count += 1.0;
-                const long long n_rec = recorded_before(S, gstep) - recorded_before(S, S.first_step);
-                for (int i = lane; i < d; i += 32) {
-                    const double x = us[i], m0 = C.mom_mean[c * d + i];
-                    const double delta = x - m0, m1 = m0 + delta / count;
-                    C.mom_mean[c * d + i] = m1;
-                    C.mom_m2[c * d + i] += delta * (x - m1);
-                    if (C.trace && n_rec < C.n_record) C.trace[(c * C.n_record + n_rec) * d + i] = x;
-                }
-            }
-        }
-        for (int i = lane; i < d; i += 32) C.u[c * d + i] = us[i];
-        if (lane == 0) {
-            C.phi[c] = phi_u;
-            C.mom_count[c] = count;
-#pragma unroll
-            for (int k = 0; k < CNT_N; ++k) C.counters[c * CNT_N + k] += cnt[k];
-        }
-        __syncwarp();
-    }
+    const Group Gp{0, 32, lane_id(), FULL};
+    const BurgersWidePhiOf<CPL, NUMERICS, PADDED> phi_of{B, par, state, Gs, r2, Gp.lane};
+    for (long long c = (long long)blockIdx.x * wpc + warp; c < n_chains; c += (long long)gridDim.x * wpc)
+        burgers_advance_chain<false>(S, C, Gp, c, 0, n_steps, n_steps, SmemVec{us, vs}, phi_of);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -539,7 +573,7 @@ __global__ void __launch_bounds__(32 * TM) burgers_team_chain_kernel(const __gri
     };
     for (long long c = blockIdx.x; c < n_chains; c += gridDim.x) {
         const long long cg = S.chain_offset + c;
-        ChainRegs R = burgers_load_chain<false>(S, C, Gp, c, phi_of, true);
+        ChainRegs<LaneVec> R = burgers_load_chain<false>(S, C, Gp, c, LaneVec{}, phi_of, true);
         for (long long s = 0; s < n_steps; ++s) metropolis_step(S, C, Gp, c, cg, s, n_steps, R, phi_of, writer);
         __syncthreads();
         if (writer) burgers_store_chain<false>(S, C, lane, c, R);

@@ -79,20 +79,24 @@ cudaError_t burgers_launch_chain_queue(const BurgersDev &b, const SamplerDev &S,
     return launch(kern, grid, 32 * wpc, burgers_smem_bytes(b.N, wpc), st, b, S, C, n_chains, n_steps, chunk);
 }
 
-// wide parameter vectors: 4 warps per CTA unless the shared memory of 4 does not fit
+// wide parameter vectors: CTAs of 4 warps (one per SM sub-partition) unless the batch is tiny, halved while
+// their shared memory exceeds 200 KB
+static int burgers_wide_warps(int N, int d, long long n) {
+    int wpc = n >= 4 * 148 ? 4 : 1;
+    while (wpc > 1 && burgers_wide_smem_bytes(N, d, wpc) > 200 * 1024) wpc /= 2;
+    return wpc;
+}
 template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_wide_forward(const BurgersDev &b, long long n, const double *u, double *G, double *phi,
                                        double *state, long long *work, cudaStream_t st) {
-    int wpc = n >= 4 * 148 ? 4 : 1;
-    while (wpc > 1 && burgers_wide_smem_bytes(b.N, b.d, wpc) > 200 * 1024) wpc /= 2;
+    const int wpc = burgers_wide_warps(b.N, b.d, n);
     return launch(burgers_wide_forward_kernel<CPL, NUM, PAD>, grid_for((n + wpc - 1) / wpc), 32 * wpc,
                   burgers_wide_smem_bytes(b.N, b.d, wpc), st, b, n, u, G, phi, state, work);
 }
 template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_wide_chain(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,
                                      long long n_steps, cudaStream_t st) {
-    int wpc = n_chains >= 4 * 148 ? 4 : 1;
-    while (wpc > 1 && burgers_wide_smem_bytes(b.N, S.d, wpc) > 200 * 1024) wpc /= 2;
+    const int wpc = burgers_wide_warps(b.N, S.d, n_chains);
     return launch(burgers_wide_chain_kernel<CPL, NUM, PAD>, grid_for((n_chains + wpc - 1) / wpc), 32 * wpc,
                   burgers_wide_smem_bytes(b.N, S.d, wpc), st, b, S, C, n_chains, n_steps);
 }

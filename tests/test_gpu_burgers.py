@@ -325,10 +325,11 @@ def test_kl_spectral_extension(G, N, m):
     assert np.all(post_sd < 1.5 * np.sqrt(lam[3:]))
 
 
-@pytest.mark.parametrize("N,m,numerics", [(128, 61, "exact"), (100, 125, "exact"), (256, 61, "fused")])
+@pytest.mark.parametrize("N,m,numerics", [(128, 61, "exact"), (100, 125, "exact"), (256, 61, "fused"),
+                                            (64, 30, "exact"), (64, 30, "fused")])   # d = 33: lane 0 holds u_0 and u_32
 def test_kl_prior_beyond_one_warp_of_parameters(G, N, m, numerics):
     """The wide path (32 < d <= 256: parameter vector, proposal and absolute parameters in shared memory;
-    include/ipmcmc.h IPMCMC_MAX_DIM_WIDE): a truncated KL prior with m = 61 / 125 modes.  Forward solves against
+    include/ipmcmc.h IPMCMC_MAX_DIM_WIDE): a truncated KL prior with m = 30 / 61 / 125 modes.  Forward solves against
     the oracle (whose KL initial condition is pinned to the reference's solver by burgers_kl_*.npz), a pCN and a
     box-constrained RW chain replayed with injected noise (every decision), and free-running chains against the
     oracle driven by the engine's own Philox noise; on-device moments against the recorded trace."""
