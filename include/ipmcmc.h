@@ -260,6 +260,55 @@ int ipmcmc_pool_moments(int64_t n_chains, int32_t dim, const double *mom_count_d
                         int64_t scratch_bytes, void *stream);
 
 /* --------------------------------------------------------------------------------------------
+ * Convergence diagnostics of a recorded trace, computed on the device for every chain of a batch.
+ *   replaces stats.integrated_autocorr_time / stats.ess_multichain called per chain on the host, and adds
+ *   split-R-hat (BDA3 section 11.4) and multi-chain ESS (BDA3 section 11.5); the estimators are restated
+ *   in NumPy in ip_mcmc_b200/stats.py (integrated_autocorr_time, split_rhat, multichain_ess).
+ * The trace is [n_chains, n_draws, dim] as ipmcmc_run writes it, with rows contiguous and chains
+ * `chain_stride` >= n_draws*dim doubles apart (a view trace[:, burn:] needs no copy).  The split
+ * estimators use the first and the last h = n_draws/2 draws of each chain as m = 2*n_chains sequences
+ * (n_draws >= 4).  Every result is deterministic: its summation order depends on (n_chains, n_draws, dim)
+ * only, not on the device, the launch geometry or whether scratch is supplied.
+ * scratch_dev: caller-owned device scratch of ipmcmc_diag_scratch_bytes(n_chains, dim, n_lags) bytes (n_lags
+ * the largest lag block the caller asks for; 0 for seqstats only), or NULL: a stream-ordered allocation is
+ * made and freed inside the call.
+ * ------------------------------------------------------------------------------------------ */
+int64_t ipmcmc_diag_scratch_bytes(int64_t n_chains, int32_t dim, int64_t n_lags);
+/* Per-chain integrated autocorrelation time with Geyer's initial-positive-sequence cut-off
+ * (stats.integrated_autocorr_time): tau_dev [n_chains, dim].  A constant series gives
+ * 1 + 4*floor((n_draws-1)/2), as the host's all-ones autocorrelation does.  One warp per series. */
+int ipmcmc_diag_tau(int64_t n_chains, int64_t n_draws, int32_t dim, const double *trace_dev,
+                    int64_t chain_stride, double *tau_dev, void *stream);
+/* Split-sequence statistics per parameter j (BDA3 section 11.4): seqstats_dev [dim, 4] =
+ * (m, mean of the sequence means, M2 = sum of squared deviations of the sequence means, sum of the
+ * sequence variances s_s^2 with ddof = 1).  Rows of several batches merge with Chan's formula
+ * (ip_mcmc_b200/parallel.py:merge_seqstats). */
+int ipmcmc_diag_seqstats(int64_t n_chains, int64_t n_draws, int32_t dim, const double *trace_dev,
+                         int64_t chain_stride, double *seqstats_dev, void *scratch_dev,
+                         int64_t scratch_bytes, void *stream);
+/* Variogram sums (BDA3 section 11.5) for the lags t in [lag0, lag0 + n_lags), lag0 + n_lags <= h:
+ *   vsum_dev[j*vsum_ld + (t - lag0)] = sum_s sum_{i=t}^{h-1} (psi_{s,i} - psi_{s,i-t})^2
+ * over the split sequences psi_s.  Parameters with done_dev[j] != 0 are skipped (their row is not
+ * written); done_dev may be NULL.  Sums of several batches add. */
+int ipmcmc_diag_variogram(int64_t n_chains, int64_t n_draws, int32_t dim, const double *trace_dev,
+                          int64_t chain_stride, int64_t lag0, int64_t n_lags, const int32_t *done_dev,
+                          double *vsum_dev, int64_t vsum_ld, void *scratch_dev, int64_t scratch_bytes,
+                          void *stream);
+/* Truncated autocorrelation sum and final estimates from seqstats_dev [dim, 4] and the variogram sums
+ * vsum_dev[j*vsum_ld + t] of the lags 1 <= t < lag_end (lag_end <= h); called after each block of lags
+ * with a growing lag_end, the last call with lag_end = h.  rho_t = 1 - V_t/(2 var+), V_t = vsum_t/(m(h-t)),
+ * var+ = (h-1)/h W + B/h, W = sum s_s^2/m, B = h/(m-1) M2.  With S = 0, t = 1:
+ *   S += rho_t; stop if t+2 > h-1 or rho_{t+1} + rho_{t+2} < 0; else S += rho_{t+1}, t += 2, repeat.
+ * state_dev [2*dim] (zero before the first call) carries the loop between calls, which pauses where a
+ * lag it needs is not summed yet; done_dev [dim] int32 (zero before the first call) is set when a
+ * parameter's loop ends, and then out_dev [3*dim] = (R-hat = sqrt(var+/W), n_eff = m h/(1 + 2S), T = t)
+ * for it.  IEEE arithmetic throughout: all sequences constant give NaN, constant ones at different
+ * values inf. */
+int ipmcmc_diag_truncate(int64_t n_draws, int32_t dim, const double *seqstats_dev, const double *vsum_dev,
+                         int64_t vsum_ld, int64_t lag_end, double *state_dev, int32_t *done_dev,
+                         double *out_dev, void *stream);
+
+/* --------------------------------------------------------------------------------------------
  * Host-buffer entry point -- what a non-Python binding of MCMCSampler.run (sampler.py:12-33) calls, and
  * what bench.py times as `e2e_c_abi`: copies u0 (and the Lorenz IC) host->device, runs n_steps with the
  * SAME kernels and scheduler as the device-buffer path (dynamic step scheduler where it applies), copies

@@ -12,7 +12,8 @@ from .potential import EvolutionPotential
 from .distribution import GaussianDistribution
 from .forward import BurgersFVM, Lorenz96Moments
 from .engine import Problem, ChainBatch, SamplerSpec, fp64_peak_tflops
-from . import stats, parallel, studies
+from . import stats, parallel, studies, diagnostics
+from .diagnostics import chain_diagnostics
 
 # the stale name the reference's scripts import (lorenz_mcmc.py:6-10, burgers_mcmc.py:4-8)
 pCNProposer = ConstSteppCNProposer
@@ -20,4 +21,5 @@ pCNProposer = ConstSteppCNProposer
 __all__ = ["MCMCSampler", "ConstStepStandardRWProposer", "VarStepStandardRWProposer", "ConstSteppCNProposer",
            "VarSteppCNProposer", "pCNProposer", "StandardRWAccepter", "pCNAccepter", "CountedAccepter",
            "ConstrainAccepter", "BoxConstraint", "EvolutionPotential", "GaussianDistribution", "BurgersFVM",
-           "Lorenz96Moments", "Problem", "ChainBatch", "SamplerSpec", "fp64_peak_tflops", "stats", "parallel", "studies"]
+           "Lorenz96Moments", "Problem", "ChainBatch", "SamplerSpec", "fp64_peak_tflops", "stats", "parallel", "studies", "diagnostics",
+           "chain_diagnostics"]

@@ -82,6 +82,14 @@ SYMBOLS = {
                                       C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "ipmcmc_sample_host": (C.c_int, [C.c_void_p, C.POINTER(SamplerDesc), C.c_int64, C.c_int64, C.POINTER(HostIO),
                                      C.c_void_p]),
+    "ipmcmc_diag_scratch_bytes": (C.c_int64, [C.c_int64, C.c_int32, C.c_int64]),
+    "ipmcmc_diag_tau": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "ipmcmc_diag_seqstats": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                       C.c_int64, C.c_void_p]),
+    "ipmcmc_diag_variogram": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
+                                        C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    "ipmcmc_diag_truncate": (C.c_int, [C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_void_p]),
     "ipmcmc_histogram_accumulate": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_void_p]),
     "ipmcmc_lorenz_rhs": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,

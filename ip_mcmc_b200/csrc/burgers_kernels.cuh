@@ -379,16 +379,6 @@ struct BurgersWidePhiOf {
     }
 };
 
-// sum over the warp in a fixed order (lane tree), the same bits on every lane
-__device__ __forceinline__ double warp_sum_fixed(double v) {
-#pragma unroll
-    for (int off = 1; off < 32; off *= 2) {
-        const double o = __shfl_xor_sync(FULL, v, off);
-        v = (lane_id() & off) ? o + v : v + o;
-    }
-    return v;
-}
-
 // The chain's parameter vector u and its proposal v in shared memory, component i on lane i % 32 (d > 32).
 // The Welford moments are updated in place in global memory, their count is kept in a register.
 struct SmemVec {

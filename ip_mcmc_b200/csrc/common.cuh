@@ -43,6 +43,27 @@ __device__ __forceinline__ double shfl(double v, int src, unsigned mask = FULL) 
 __device__ __forceinline__ double shfl_up1(double v) { return __shfl_up_sync(FULL, v, 1); }
 __device__ __forceinline__ double shfl_down1(double v) { return __shfl_down_sync(FULL, v, 1); }
 
+// sum over the warp in a fixed order (lane tree), the same bits on every lane
+__device__ __forceinline__ double warp_sum_fixed(double v) {
+#pragma unroll
+    for (int off = 1; off < 32; off *= 2) {
+        const double o = __shfl_xor_sync(FULL, v, off);
+        v = (lane_id() & off) ? o + v : v + o;
+    }
+    return v;
+}
+
+// (count, mean, M2) and Chan et al.'s merge of two such triples
+struct Mom3 {
+    double n, mean, m2;
+};
+__device__ __forceinline__ Mom3 chan_merge(const Mom3 &a, const Mom3 &b) {
+    const double nt = a.n + b.n;
+    if (!(nt > 0.0)) return Mom3{0.0, 0.0, 0.0};
+    const double delta = b.mean - a.mean;
+    return Mom3{nt, a.mean + delta * (b.n / nt), (a.m2 + b.m2) + delta * delta * (a.n * b.n / nt)};
+}
+
 // |x| as an ordered 64-bit integer key: IEEE-754 ordering of non-negative doubles equals the
 // ordering of their bit patterns.  Kept in integer registers on purpose -- a round trip through
 // double makes the compiler re-materialise fabs as a DADD on the (precious) fp64 pipe.

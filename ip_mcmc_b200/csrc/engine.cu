@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "burgers_launch.cuh"
+#include "diag.cuh"
 #include "lorenz_kernels.cuh"
 
 using namespace ipmcmc;
@@ -480,16 +481,6 @@ extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const
 constexpr int POOL_THREADS = 256;
 constexpr int POOL_CHUNK = 2048;
 
-struct Mom3 {
-    double n, mean, m2;
-};
-__device__ __forceinline__ Mom3 chan_merge(const Mom3 &a, const Mom3 &b) {
-    const double nt = a.n + b.n;
-    if (!(nt > 0.0)) return Mom3{0.0, 0.0, 0.0};
-    const double delta = b.mean - a.mean;
-    return Mom3{nt, a.mean + delta * (b.n / nt), (a.m2 + b.m2) + delta * delta * (a.n * b.n / nt)};
-}
-
 __global__ void __launch_bounds__(POOL_THREADS) pool_partial_kernel(long long n_chains, int d,
                                                                     const double *__restrict__ cnt,
                                                                     const double *__restrict__ mean,
@@ -595,6 +586,128 @@ extern "C" int ipmcmc_pool_moments(int64_t n_chains, int32_t dim, const double *
     const int rc = pool_launch(n_chains, dim, mom_count_dev, mom_mean_dev, mom_m2_dev, (const long long *)counters_dev, pooled_dev, tmp, st);
     cudaFreeAsync(tmp, st);
     return rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// convergence diagnostics of a recorded trace (diag.cuh)
+// ------------------------------------------------------------------------------------------------
+static int diag_check(int64_t n_chains, int64_t n, int32_t dim, const double *trace, int64_t stride, int64_t n_min) {
+    if (n_chains < 1) return fail(IPMCMC_EINVAL, "n_chains=%lld", (long long)n_chains);
+    if (n < n_min) return fail(IPMCMC_EINVAL, "n_draws=%lld (at least %lld)", (long long)n, (long long)n_min);
+    if (n > 2147483647LL) return fail(IPMCMC_EUNSUPPORTED, "n_draws=%lld (at most 2^31 - 1)", (long long)n);
+    if (dim < 1 || dim > IPMCMC_MAX_DIM_WIDE) return fail(IPMCMC_EINVAL, "dim=%d", dim);
+    if (stride < n * dim) return fail(IPMCMC_EINVAL, "chain_stride=%lld < n_draws*dim=%lld", (long long)stride, (long long)(n * dim));
+    if (!trace) return fail(IPMCMC_EINVAL, "NULL trace");
+    return 0;
+}
+
+static long long seq_blocks(long long M) { return (M + SEQ_CHUNK - 1) / SEQ_CHUNK; }
+static long long vario_blocks(long long M) { const long long c = vario_chunk(M); return (M + c - 1) / c; }
+
+extern "C" int64_t ipmcmc_diag_scratch_bytes(int64_t n_chains, int32_t dim, int64_t n_lags) {
+    if (n_chains < 1 || dim < 1 || n_lags < 0) return 0;
+    const long long a = seq_blocks(n_chains) * dim * 4, b = vario_blocks(n_chains) * dim * n_lags;
+    return (int64_t)((a > b ? a : b) * sizeof(double));
+}
+
+// runs body(scratch) on the caller's scratch (checked against need) or a stream-ordered allocation
+template <class F>
+static int with_scratch(void *scratch, int64_t scratch_bytes, int64_t need, cudaStream_t st, const F &body) {
+    if (scratch) {
+        if (scratch_bytes < need) return fail(IPMCMC_EINVAL, "diagnostics scratch: %lld bytes given, %lld needed", (long long)scratch_bytes, (long long)need);
+        return body(scratch);
+    }
+    void *tmp = nullptr;
+    CUDA_TRY(cudaMallocAsync(&tmp, (size_t)need, st));
+    const int rc = body(tmp);
+    cudaFreeAsync(tmp, st);
+    return rc;
+}
+
+extern "C" int ipmcmc_diag_tau(int64_t n_chains, int64_t n_draws, int32_t dim, const double *trace_dev, int64_t chain_stride,
+                               double *tau_dev, void *stream) {
+    if (int rc = diag_check(n_chains, n_draws, dim, trace_dev, chain_stride, 1)) return rc;
+    if (!tau_dev) return fail(IPMCMC_EINVAL, "NULL tau_dev");
+    const long long series_bytes = n_draws * (long long)sizeof(double);
+    const bool staged = series_bytes <= DIAG_SMEM;
+    const int warps = staged ? (int)(DIAG_SMEM / series_bytes < 8 ? DIAG_SMEM / series_bytes : 8) : 8;
+    const size_t smem = staged ? (size_t)(warps * series_bytes) : 0;
+    const unsigned grid = (unsigned)grid_for((n_chains * dim + warps - 1) / warps);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (staged) {
+        CUDA_TRY(cudaFuncSetAttribute(diag_tau_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM));
+        diag_tau_kernel<true><<<grid, 32 * warps, smem, st>>>(n_chains, n_draws, dim, trace_dev, chain_stride, tau_dev);
+    } else {
+        diag_tau_kernel<false><<<grid, 32 * warps, 0, st>>>(n_chains, n_draws, dim, trace_dev, chain_stride, tau_dev);
+    }
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int ipmcmc_diag_seqstats(int64_t n_chains, int64_t n_draws, int32_t dim, const double *trace_dev,
+                                    int64_t chain_stride, double *seqstats_dev, void *scratch_dev, int64_t scratch_bytes,
+                                    void *stream) {
+    if (int rc = diag_check(n_chains, n_draws, dim, trace_dev, chain_stride, 4)) return rc;
+    if (!seqstats_dev) return fail(IPMCMC_EINVAL, "NULL seqstats_dev");
+    const long long nb = seq_blocks(n_chains);
+    if (nb > 2147483647LL) return fail(IPMCMC_EUNSUPPORTED, "n_chains=%lld", (long long)n_chains);
+    cudaStream_t st = (cudaStream_t)stream;
+    return with_scratch(scratch_dev, scratch_bytes, (int64_t)(nb * dim * 4 * sizeof(double)), st, [&](void *s) {
+        double *part = (double *)s;
+        diag_seq_partial_kernel<<<dim3((unsigned)nb, (unsigned)dim), DIAG_WARPS * 32, 0, st>>>(n_chains, n_draws, dim, trace_dev,
+                                                                                              chain_stride, part);
+        CUDA_TRY(cudaGetLastError());
+        diag_seq_final_kernel<<<1, 64, 0, st>>>((int)nb, dim, part, seqstats_dev);
+        CUDA_TRY(cudaGetLastError());
+        return 0;
+    });
+}
+
+extern "C" int ipmcmc_diag_variogram(int64_t n_chains, int64_t n_draws, int32_t dim, const double *trace_dev,
+                                     int64_t chain_stride, int64_t lag0, int64_t n_lags, const int32_t *done_dev,
+                                     double *vsum_dev, int64_t vsum_ld, void *scratch_dev, int64_t scratch_bytes, void *stream) {
+    if (int rc = diag_check(n_chains, n_draws, dim, trace_dev, chain_stride, 4)) return rc;
+    const long long h = n_draws / 2;
+    if (lag0 < 0 || n_lags < 1 || lag0 + n_lags > h)
+        return fail(IPMCMC_EINVAL, "lags [%lld, %lld) outside [0, h=%lld)", (long long)lag0, (long long)(lag0 + n_lags), h);
+    if (!vsum_dev || vsum_ld < n_lags) return fail(IPMCMC_EINVAL, "vsum_dev=%p vsum_ld=%lld", (void *)vsum_dev, (long long)vsum_ld);
+    const long long groups = (n_lags + 31) / 32;
+    if (groups > 65535) return fail(IPMCMC_EUNSUPPORTED, "n_lags=%lld (at most %d per call)", (long long)n_lags, 65535 * 32);
+    const long long nb = vario_blocks(n_chains);
+    const bool staged = (long long)DIAG_WARPS * h * (long long)sizeof(double) <= DIAG_SMEM;
+    cudaStream_t st = (cudaStream_t)stream;
+    return with_scratch(scratch_dev, scratch_bytes, (int64_t)(nb * dim * n_lags * sizeof(double)), st, [&](void *s) {
+        double *part = (double *)s;
+        const dim3 grid((unsigned)nb, (unsigned)groups, (unsigned)dim);
+        if (staged) {
+            CUDA_TRY(cudaFuncSetAttribute(diag_vario_partial_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DIAG_SMEM));
+            diag_vario_partial_kernel<true><<<grid, DIAG_WARPS * 32, (size_t)(DIAG_WARPS * h * sizeof(double)), st>>>(
+                n_chains, n_draws, dim, trace_dev, chain_stride, lag0, n_lags, done_dev, part);
+        } else {
+            diag_vario_partial_kernel<false><<<grid, DIAG_WARPS * 32, 0, st>>>(n_chains, n_draws, dim, trace_dev, chain_stride,
+                                                                              lag0, n_lags, done_dev, part);
+        }
+        CUDA_TRY(cudaGetLastError());
+        const long long fb = (n_lags + 127) / 128;
+        diag_vario_final_kernel<<<dim3((unsigned)(fb < 1024 ? fb : 1024), (unsigned)dim), 128, 0, st>>>((int)nb, dim, n_lags, part,
+                                                                                                     done_dev, vsum_dev, vsum_ld);
+        CUDA_TRY(cudaGetLastError());
+        return 0;
+    });
+}
+
+extern "C" int ipmcmc_diag_truncate(int64_t n_draws, int32_t dim, const double *seqstats_dev, const double *vsum_dev,
+                                    int64_t vsum_ld, int64_t lag_end, double *state_dev, int32_t *done_dev, double *out_dev,
+                                    void *stream) {
+    const long long h = n_draws / 2;
+    if (n_draws < 4 || dim < 1 || dim > IPMCMC_MAX_DIM_WIDE) return fail(IPMCMC_EINVAL, "n_draws=%lld dim=%d", (long long)n_draws, dim);
+    if (lag_end < 1 || lag_end > h || vsum_ld < lag_end)
+        return fail(IPMCMC_EINVAL, "lag_end=%lld vsum_ld=%lld (h=%lld)", (long long)lag_end, (long long)vsum_ld, h);
+    if (!seqstats_dev || !vsum_dev || !state_dev || !done_dev || !out_dev) return fail(IPMCMC_EINVAL, "NULL argument");
+    diag_truncate_kernel<<<1, 64, 0, (cudaStream_t)stream>>>(h, dim, seqstats_dev, vsum_dev, vsum_ld, lag_end, state_dev,
+                                                             done_dev, out_dev);
+    CUDA_TRY(cudaGetLastError());
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -1,8 +1,10 @@
 """Multi-GPU plumbing: chains are independent, so ranks own contiguous blocks of GLOBAL chain ids
 (Philox is keyed by the global id, results do not depend on the GPU count) and exchange nothing
-while sampling.  The only collective is the final reduction of pooled moments and counters
+while sampling.  The only collective of a run is the final reduction of pooled moments and counters
 (SURVEY.md section 8(e)): ONE all-gather of 2d+7 doubles per rank followed by a local Chan merge
-(latency-bound; NCCL over NVLink on the GPU box, gloo in the CPU tests)."""
+(latency-bound; NCCL over NVLink on the GPU box, gloo in the CPU tests).  Convergence diagnostics
+(diagnostics.chain_diagnostics) merge their split-sequence statistics the same way and add one all-gather
+of the variogram sums per block of lags."""
 import torch
 import torch.distributed as dist
 
@@ -36,6 +38,44 @@ def merge_pooled(allp, d):
     mean_tot = torch.where(n_tot > 0, (n * mean).sum(0) / torch.clamp(n_tot, min=1.0), torch.zeros_like(mean[0]))
     m2_tot = (m2 + n * (mean - mean_tot) ** 2).sum(0)
     return torch.cat([n_tot, mean_tot, m2_tot, allp[:, 1 + 2 * d:].sum(0)])
+
+
+def distributed(group=None):
+    """True when a process group with more than one rank is initialised."""
+    return dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+
+
+def allgather(x, group=None):
+    """[world, *x.shape]: x of every rank in rank order (ONE all-gather); [1, *x.shape] without a group."""
+    if not distributed(group):
+        return x.unsqueeze(0).clone()
+    world = dist.get_world_size(group)
+    out = torch.empty((world * x.numel(),), dtype=x.dtype, device=x.device)
+    dist.all_gather_into_tensor(out, x.contiguous().reshape(-1), group=group)
+    return out.reshape((world,) + tuple(x.shape))
+
+
+def merge_seqstats(alls):
+    """Split-sequence statistics of several batches [world, d, 4] = (m, mean of the sequence means, M2 of the
+    sequence means, sum of the sequence variances) (ipmcmc_diag_seqstats) -> [d, 4] of all their sequences:
+    Chan's merge in rank order, the sums of variances added in rank order, so every rank gets the same bits."""
+    r = alls[0].clone()
+    for b in alls[1:]:
+        n = r[:, 0] + b[:, 0]
+        delta = b[:, 1] - r[:, 1]
+        mean = r[:, 1] + delta * (b[:, 0] / n)
+        m2 = (r[:, 2] + b[:, 2]) + delta * delta * (r[:, 0] * b[:, 0] / n)
+        r = torch.stack([n, mean, m2, r[:, 3] + b[:, 3]], dim=1)
+    return r
+
+
+def merge_sums(alls):
+    """Sums of several batches [world, ...] (variogram sums of one lag block, ESS totals) -> their sum,
+    added in rank order."""
+    r = alls[0].clone()
+    for b in alls[1:]:
+        r = r + b
+    return r
 
 
 def max_over_ranks(x, device, group=None):

@@ -15,6 +15,7 @@ import torch
 
 from . import _lib
 from . import accepter as _acc
+from . import diagnostics as _diag
 from . import stats as _stats
 from .engine import ChainBatch, SamplerSpec, F64
 from .potential import EvolutionPotential
@@ -56,7 +57,7 @@ class MCMCSampler:
         return spec, pot, a
 
     def run(self, u_0, n_samples, burn_in=1000, sample_interval=200, n_chains=None, chain_offset=0,
-            steps_per_launch=None, return_device=False, recompute_phi_u=None, scheduler=None, out=None, phi_0=None):
+            steps_per_launch=None, return_device=False, recompute_phi_u=None, scheduler=None, out=None, phi_0=None, diagnostics=False):
         """Same step accounting as the reference (sampler.py:18-28): max(0, burn_in - interval)
         unrecorded steps, then n_samples * interval steps recording every interval-th state.
 
@@ -66,9 +67,13 @@ class MCMCSampler:
         n_chains * n_samples * d float64; a PINNED torch tensor makes the device->host copy a single DMA).
         `phi_0`: Phi(u_0) per chain when it is known -- `last_run["phi"]` of the run that ended in u_0 --
         so that a continued run does not pay one more forward solve per chain (deterministic models only).
+        `diagnostics`: fill `last_run["diagnostics"]` with diagnostics.chain_diagnostics of the device trace (every
+        chain; over all ranks of an initialised process group) before it is copied out; the samples are unchanged.
         """
         if sample_interval < 1:
             raise ValueError("sample_interval must be >= 1")
+        if diagnostics and n_samples < 4:
+            raise ValueError("diagnostics=True needs at least 4 samples per chain (split-R-hat), got %d" % n_samples)
         pre = max(0, burn_in - sample_interval)
         total = pre + n_samples * sample_interval
         spec, pot, a = self._compile(total, burn_in, sample_interval, recompute_phi_u)
@@ -112,6 +117,8 @@ class MCMCSampler:
                              h2d_bytes=chains.h2d_bytes, u=chains.u, phi=chains.phi)
         cn = self.last_run["counters"]
         _acc.credit_counters(a, cn["calls"], cn["accepts"], cn["constraint_rejects"])
+        if diagnostics:
+            self.last_run["diagnostics"] = _diag.chain_diagnostics(trace)
         if return_device:
             return trace[0] if single else trace
         if out is not None:

@@ -91,6 +91,58 @@ def ess_multichain(traces):
     return float(per.sum()), per
 
 
+def split_sequences(traces):
+    """traces [M, n, d] -> the 2M split sequences [2M, h, d], h = n // 2: the first and the last h draws of
+    each chain (the middle draw of an odd n is dropped), sequence 2c and 2c+1 from chain c."""
+    x = np.asarray(traces, dtype=np.float64)
+    if x.ndim != 3 or x.shape[1] < 4:
+        raise ValueError("traces must be [n_chains, n >= 4, d], got %s" % (x.shape,))
+    h = x.shape[1] // 2
+    return np.stack([x[:, :h], x[:, x.shape[1] - h:]], axis=1).reshape(-1, h, x.shape[2])
+
+
+def _split_var_plus(psi):
+    """(W, var+) of split sequences psi [m, h, d] (BDA3 section 11.4)."""
+    m, h = psi.shape[0], psi.shape[1]
+    means = psi.mean(axis=1)
+    W = psi.var(axis=1, ddof=1).mean(axis=0)
+    B = h / (m - 1) * ((means - means.mean(axis=0)) ** 2).sum(axis=0)
+    return W, (h - 1) / h * W + B / h
+
+
+def split_rhat(traces):
+    """Split-R-hat (BDA3 section 11.4) of traces [M, n, d] -> [d]: sqrt(var+ / W) over the 2M half-chains.
+    All sequences constant gives NaN (0/0), constant sequences at different values inf."""
+    with np.errstate(divide="ignore", invalid="ignore"):
+        W, var_plus = _split_var_plus(split_sequences(traces))
+        return np.sqrt(var_plus / W)
+
+
+def multichain_ess(traces):
+    """Multi-chain effective sample size (BDA3 section 11.5, variogram form) of traces [M, n, d] on the split
+    sequences -> (n_eff [d], T [d]).  rho_t = 1 - V_t / (2 var+), V_t the mean squared difference of draws t
+    apart; the sum of rho_t runs over t = 1, 2, ... and stops at the first odd T with
+    rho_{T+1} + rho_{T+2} < 0 (or T + 2 > h - 1); n_eff = m h / (1 + 2 S)."""
+    psi = split_sequences(traces)
+    m, h, d = psi.shape
+    n_eff, cutoff = np.empty(d), np.empty(d, dtype=np.int64)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        _, var_plus = _split_var_plus(psi)
+        for j in range(d):
+            def rho(t):
+                V = ((psi[:, t:, j] - psi[:, :h - t, j]) ** 2).sum() / (m * (h - t))
+                return 1.0 - V / (2.0 * var_plus[j])
+            S, t = 0.0, 1
+            while True:
+                S += rho(t)
+                if t + 2 > h - 1 or rho(t + 1) + rho(t + 2) < 0:
+                    break
+                S += rho(t + 1)
+                t += 2
+            n_eff[j], cutoff[j] = m * h / (1.0 + 2.0 * S), t
+    return n_eff, cutoff
+
+
 def usable_samples(n, burn_in, tau0):
     """M = (N - b) / tau_0 (report/burgers.org:43-45)."""
     return (n - burn_in) / max(tau0, 1)
