@@ -244,6 +244,38 @@ typedef struct ipmcmc_chain_buffers {
 int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipmcmc_chain_buffers *b,
                int64_t n_chains, int64_t n_steps, void *stream);
 
+/* --------------------------------------------------------------------------------------------
+ * Replica exchange (parallel tempering) for Burgers chains.  Not in the reference.
+ * A tempered batch is n_ladders x K chains, ladder-major: local chain c = l*K + k is rung k of ladder l
+ * (global id chain_offset + c; chain_offset a multiple of K, so a shard owns whole ladders).
+ *
+ * ipmcmc_run_tempered: ipmcmc_run with the likelihood of chain c tempered by inv_temp_dev[c] (t, [n_chains]):
+ *   a = exp((t*Phi(u) + reg_u) - (t*Phi(v) + reg_v)),  accepted = a > U
+ * reg is the RW regulariser 0.5*||L w||^2 (0 for pCN) and is not tempered; Phi itself stays untempered in
+ * phi_dev and the step log.  t = 1 gives ipmcmc_run's results bit for bit.  Lorenz chains: IPMCMC_EUNSUPPORTED
+ * (their Phi depends on the carried initial condition).
+ * ------------------------------------------------------------------------------------------ */
+int ipmcmc_run_tempered(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipmcmc_chain_buffers *b,
+                        const double *inv_temp_dev, int64_t n_chains, int64_t n_steps, void *stream);
+/* One swap round r (>= 0) between adjacent rungs, run after global step (r+1)*swap_interval.  It proposes the
+ * pairs (k, k+1) with k = r (mod 2) in every ladder and swaps iff
+ *   exp((t_k - t_{k+1}) * (Phi_k - Phi_{k+1})) > U      (strict; NaN never swaps)
+ * U = Philox4x32-10 keyed (seed lo, global id of slot k), counter (r lo, r hi, 0xFFFFFFFE, seed hi) -- a slot
+ * no Metropolis draw uses -- or inject_u_dev[l*(K-1) + k] when inject_u_dev [n_ladders, K-1] is not NULL.
+ * On a swap the rows of u_dev [n_ladders*K, dim], the entries of phi_dev and the rows of replica_dev move;
+ * Welford moments, counters and traces stay with the slot.
+ *   replica_dev      [n_ladders*K, 2] int32 (replica id, direction); start from (k, 0).  After the swaps slot 0
+ *                    gets direction +1, incrementing round_trips_dev[l] if it was -1, and slot K-1 gets -1
+ *                    (in the rounds that propose pair (0,1), resp. pair (K-2,K-1)).
+ *   swap_counts_dev  [n_ladders, K-1, 2] int64 (attempts, accepts) per adjacent pair, accumulated
+ *   round_trips_dev  [n_ladders] int64, accumulated
+ * Arguments are checked before any CUDA call: K >= 2, n_ladders >= 1, 1 <= dim <= 256, round >= 0,
+ * chain_offset % K == 0, global ids below 2^32, and every pointer but inject_u_dev non-NULL. */
+int ipmcmc_swap_replicas(int64_t n_ladders, int32_t ladder_size, int32_t dim, double *u_dev, double *phi_dev,
+                         const double *inv_temp_dev, uint64_t seed, int64_t chain_offset, int64_t round,
+                         const double *inject_u_dev, int32_t *replica_dev, int64_t *swap_counts_dev,
+                         int64_t *round_trips_dev, void *stream);
+
 /* Pool per-chain Welford moments and counters of n_chains chains into
  *   pooled_dev[0] = n, [1..d] = mean, [1+d..2d] = M2, then the 6 counters as doubles
  * (2d + 7 doubles) with Chan's parallel merge as a fixed tree (deterministic; two small launches whose

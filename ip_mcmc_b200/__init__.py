@@ -14,6 +14,8 @@ from .forward import BurgersFVM, Lorenz96Moments
 from .engine import Problem, ChainBatch, SamplerSpec, fp64_peak_tflops
 from . import stats, parallel, studies, diagnostics
 from .diagnostics import chain_diagnostics
+from . import tempering
+from .tempering import ParallelTemperingSampler, geometric_inv_temps
 
 # the stale name the reference's scripts import (lorenz_mcmc.py:6-10, burgers_mcmc.py:4-8)
 pCNProposer = ConstSteppCNProposer
@@ -22,4 +24,4 @@ __all__ = ["MCMCSampler", "ConstStepStandardRWProposer", "VarStepStandardRWPropo
            "VarSteppCNProposer", "pCNProposer", "StandardRWAccepter", "pCNAccepter", "CountedAccepter",
            "ConstrainAccepter", "BoxConstraint", "EvolutionPotential", "GaussianDistribution", "BurgersFVM",
            "Lorenz96Moments", "Problem", "ChainBatch", "SamplerSpec", "fp64_peak_tflops", "stats", "parallel", "studies", "diagnostics",
-           "chain_diagnostics"]
+           "chain_diagnostics", "tempering", "ParallelTemperingSampler", "geometric_inv_temps"]

@@ -77,6 +77,11 @@ SYMBOLS = {
                                  C.c_void_p, C.c_void_p]),
     "ipmcmc_run": (C.c_int, [C.c_void_p, C.POINTER(SamplerDesc), C.POINTER(ChainBuffers), C.c_int64,
                              C.c_int64, C.c_void_p]),
+    "ipmcmc_run_tempered": (C.c_int, [C.c_void_p, C.POINTER(SamplerDesc), C.POINTER(ChainBuffers), C.c_void_p,
+                                      C.c_int64, C.c_int64, C.c_void_p]),
+    "ipmcmc_swap_replicas": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p]),
     "ipmcmc_pool_scratch_bytes": (C.c_int64, [C.c_int64, C.c_int32]),
     "ipmcmc_pool_moments": (C.c_int, [C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),

@@ -30,7 +30,7 @@ NVCC_FLAGS = CFLAGS      # (name kept for tools/)
 # is older than the unit's source or any of them
 _COMMON = ["common.cuh", "philox.cuh", "sampler.cuh", "sched.cuh", "burgers.cuh", "burgers_launch.cuh",
            os.path.join("..", "..", "include", "ipmcmc.h")]
-DEPS = {"engine.cu": _COMMON + ["diag.cuh", "lorenz.cuh", "lorenz_kernels.cuh"],
+DEPS = {"engine.cu": _COMMON + ["diag.cuh", "lorenz.cuh", "lorenz_kernels.cuh", "tempering.cuh"],
         "burgers_inst.cu": _COMMON + ["burgers_kernels.cuh", "burgers_team.cuh", "burgers_launch_impl.cuh"]}
 
 

@@ -213,7 +213,11 @@ __device__ IPMCMC_STEP_INLINE void metropolis_step(const SamplerDev &S, const Ch
         R.cnt[CNT_WORK_B] += 1;
         double reg_v = 0.0;
         if (S.accepter == IPMCMC_ACCEPT_RW) reg_v = R.x.regulariser(S, Gp, v);
-        a = exp((R.phi_u + R.reg_u) - (phi_v + reg_v));
+        // the chain's inverse temperature t tempers Phi, not the RW regulariser; Phi itself stays untempered.  t = 1
+        // (every untempered chain) multiplies exactly: the reference's exp((Phi(u)+reg_u) - (Phi(v)+reg_v)).  Read
+        // here, after the solve, rather than carried in ChainRegs: a register live across the solve moves its allocation.
+        const double t = C.inv_temp ? C.inv_temp[c] : 1.0;
+        a = exp((t * R.phi_u + R.reg_u) - (t * phi_v + reg_v));
         const double U = C.inject_u ? C.inject_u[c * n_steps + s] : draw_uniform(S.seed, (uint64_t)cg, (uint64_t)gstep);
         accepted = a > U;  // strict, un-clipped; NaN compares false (accepter.py:61-62)
         if (!isfinite(phi_v)) R.cnt[CNT_NONFINITE] += 1;

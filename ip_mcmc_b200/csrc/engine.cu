@@ -13,6 +13,7 @@
 #include "burgers_launch.cuh"
 #include "diag.cuh"
 #include "lorenz_kernels.cuh"
+#include "tempering.cuh"
 
 using namespace ipmcmc;
 
@@ -389,9 +390,13 @@ static int make_sampler(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, Sampler
     return 0;
 }
 
-extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipmcmc_chain_buffers *b,
-                          int64_t n_chains, int64_t n_steps, void *stream) {
+// ipmcmc_run (inv_temp NULL) and ipmcmc_run_tempered
+static int run_chains(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipmcmc_chain_buffers *b,
+                      const double *inv_temp, int64_t n_chains, int64_t n_steps, void *stream) {
     if (!p || !s || !b) return fail(IPMCMC_EINVAL, "NULL argument");
+    if (inv_temp && p->model == IPMCMC_MODEL_LORENZ)
+        return fail(IPMCMC_EUNSUPPORTED, "Lorenz chains cannot be tempered: Phi(u) depends on the carried initial "
+                                         "condition, so a replica swap is not a valid Metropolis move for them");
     if (n_chains <= 0 || n_steps < 0) return fail(IPMCMC_EINVAL, "n_chains=%lld n_steps=%lld", (long long)n_chains, (long long)n_steps);
     if (!b->u_dev || !b->phi_dev || !b->mom_count_dev || !b->mom_mean_dev || !b->mom_m2_dev || !b->counters_dev)
         return fail(IPMCMC_EINVAL, "chain state buffer is NULL");
@@ -417,6 +422,7 @@ extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const
     C.slot_chain = b->slot_chain_dev;
     C.n_slots = b->n_slots;
     C.sched = (long long *)b->sched_dev;
+    C.inv_temp = inv_temp;
     int chunk = b->sched_chunk > 0 ? b->sched_chunk : 1;   // steps per work item of the dynamic scheduler
     if (const char *e = getenv("IPMCMC_SCHED_CHUNK")) chunk = atoi(e) > 0 ? atoi(e) : chunk;  // experiments
     if (p->model == IPMCMC_MODEL_BURGERS) {
@@ -464,6 +470,58 @@ extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const
     LORENZ_DISPATCH(lorenz_chain_kernel, p->l.J, p->l.K, p->numerics,
                     <<<grid_for((warps + wpc - 1) / wpc), 32 * wpc, wpc * lorenz_smem_bytes(p->l.K), st>>>(
                         p->l, S, C, n_chains, n_steps));
+    return 0;
+}
+
+extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipmcmc_chain_buffers *b,
+                          int64_t n_chains, int64_t n_steps, void *stream) {
+    return run_chains(p, s, b, nullptr, n_chains, n_steps, stream);
+}
+
+extern "C" int ipmcmc_run_tempered(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipmcmc_chain_buffers *b,
+                                   const double *inv_temp_dev, int64_t n_chains, int64_t n_steps, void *stream) {
+    if (!inv_temp_dev) return fail(IPMCMC_EINVAL, "inv_temp_dev is NULL (use ipmcmc_run for untempered chains)");
+    return run_chains(p, s, b, inv_temp_dev, n_chains, n_steps, stream);
+}
+
+// ------------------------------------------------------------------------------------------------
+// replica exchange (tempering.cuh)
+// ------------------------------------------------------------------------------------------------
+extern "C" int ipmcmc_swap_replicas(int64_t n_ladders, int32_t ladder_size, int32_t dim, double *u_dev, double *phi_dev,
+                                    const double *inv_temp_dev, uint64_t seed, int64_t chain_offset, int64_t round,
+                                    const double *inject_u_dev, int32_t *replica_dev, int64_t *swap_counts_dev,
+                                    int64_t *round_trips_dev, void *stream) {
+    const int K = ladder_size;
+    if (K < 2 || n_ladders < 1) return fail(IPMCMC_EINVAL, "ladder_size=%d (at least 2) n_ladders=%lld (at least 1)", K, (long long)n_ladders);
+    if (dim < 1 || dim > IPMCMC_MAX_DIM_WIDE) return fail(IPMCMC_EINVAL, "dim=%d outside [1,%d]", dim, IPMCMC_MAX_DIM_WIDE);
+    if (round < 0) return fail(IPMCMC_EINVAL, "round=%lld < 0", (long long)round);
+    if (chain_offset < 0 || chain_offset % K != 0)
+        return fail(IPMCMC_EINVAL, "chain_offset=%lld is not a multiple of ladder_size=%d: a ladder would be split", (long long)chain_offset, K);
+    if (n_ladders > ((1LL << 32) - chain_offset) / K)
+        return fail(IPMCMC_EUNSUPPORTED, "global chain ids must lie in [0, 2^32): chain_offset=%lld n_ladders=%lld ladder_size=%d",
+                    (long long)chain_offset, (long long)n_ladders, K);
+    if (!u_dev || !phi_dev || !inv_temp_dev || !replica_dev || !swap_counts_dev || !round_trips_dev)
+        return fail(IPMCMC_EINVAL, "NULL argument");
+    SwapDev W;
+    W.n_ladders = n_ladders;
+    W.chain_offset = chain_offset;
+    W.round = round;
+    W.K = K;
+    W.d = dim;
+    W.parity = (int)(round & 1);
+    W.n_pairs = (K - W.parity) / 2;
+    W.seed = seed;
+    W.u = u_dev;
+    W.phi = phi_dev;
+    W.inv_temp = inv_temp_dev;
+    W.inject_u = inject_u_dev;
+    W.replica = replica_dev;
+    W.swap_counts = (long long *)swap_counts_dev;
+    W.round_trips = (long long *)round_trips_dev;
+    if (W.n_pairs == 0) return 0;   // K = 2, odd round: no pair
+    const long long warps = n_ladders * W.n_pairs;
+    swap_round_kernel<<<grid_for((warps + 7) / 8), 256, 0, (cudaStream_t)stream>>>(W);
+    CUDA_TRY(cudaGetLastError());
     return 0;
 }
 

@@ -39,9 +39,11 @@ __device__ __forceinline__ Philox4 draw_words(uint64_t seed, uint64_t chain, uin
                          (uint32_t)seed, (uint32_t)chain);
 }
 
-// U in [0,1): the 53-bit mapping numpy's Generator.random() uses ((x >> 11) * 2^-53).
-__device__ __forceinline__ double draw_uniform(uint64_t seed, uint64_t chain, uint64_t step) {
-    const Philox4 r = draw_words(seed, chain, step, SLOT_UNIFORM);
+// U in [0,1): the 53-bit mapping numpy's Generator.random() uses ((x >> 11) * 2^-53).  The accept uniform
+// uses SLOT_UNIFORM, the replica-exchange uniform SLOT_SWAP (tempering.cuh).
+__device__ __forceinline__ double draw_uniform(uint64_t seed, uint64_t chain, uint64_t step,
+                                               uint32_t slot = SLOT_UNIFORM) {
+    const Philox4 r = draw_words(seed, chain, step, slot);
     const uint64_t x = ((uint64_t)r.x1 << 32) | r.x0;
     return (double)(x >> 11) * 0x1.0p-53;
 }

@@ -6,7 +6,8 @@
 //                                             proposer.py:53-56,110-115 (VarStep: per-step table)
 //   w          N(0,C) draw = factor @ z       distribution.py:114-118 (numpy svd map)
 //   accept     a > U, a = exp(I(u)-I(v))      accepter.py:59-62 (strict, un-clipped, NaN rejects)
-//              I = Phi (+ 0.5||L w||^2 RW)    accepter.py:98-106, 121-122
+//              I = t*Phi (+ 0.5||L w||^2 RW)  accepter.py:98-106, 121-122; t = inverse temperature
+//                                             (replica exchange, tempering.cuh), 1 for the reference
 //   constraint reject before drawing U        accepter.py:52-55
 //   counters   calls / accepts                accepter.py:13-36
 //   recording  sampler.py:18-28 (burn-in max(0, b - si), thinning si)
@@ -41,6 +42,7 @@ struct ChainBufDev {
     const int *slot_chain;
     int n_slots;
     long long *sched;   // dynamic step scheduler scratch (int64 [3*n_chains + 2]) or nullptr
+    const double *inv_temp;  // [n_chains] inverse temperature of each chain's likelihood, or nullptr (= 1)
 };
 
 enum : int { CNT_CALLS = 0, CNT_ACCEPTS, CNT_WORK_A, CNT_WORK_B, CNT_NONFINITE, CNT_CONSTRAINT, CNT_N };

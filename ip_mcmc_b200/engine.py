@@ -229,6 +229,9 @@ class ChainBatch:
         self.launches = 0
         self.placement = None
         self._work_prev = None
+        # optional [n_chains] float64 cuda tensor: inverse temperature of each chain's likelihood (replica
+        # exchange, tempering.py); None runs the untempered kernel path (ipmcmc_run)
+        self.inv_temp = None
         self.sched = None          # scratch of the dynamic step scheduler (Burgers N <= 1024, Lorenz)
         self.sched_chunk = 0       # Metropolis steps per work item; 0 = automatic (Burgers: min(4, max(1, n_steps // 64)); Lorenz: 1)
         if problem.kind == _lib.MODEL_LORENZ:
@@ -282,8 +285,41 @@ class ChainBatch:
                 b.n_slots = pl.n_slots
             if pl.active:
                 self._work_prev = self.counters[:, 2].clone()
-        check(lib.ipmcmc_run(self.problem.handle, C.byref(s), C.byref(b), self.n, int(n_steps), _stream()))
+        if self.inv_temp is None:
+            check(lib.ipmcmc_run(self.problem.handle, C.byref(s), C.byref(b), self.n, int(n_steps), _stream()))
+        else:
+            check(lib.ipmcmc_run_tempered(self.problem.handle, C.byref(s), C.byref(b), _ptr(self._inv_temp_checked()),
+                                          self.n, int(n_steps), _stream()))
         self.step += int(n_steps)
+        self.launches += 1
+
+    def _inv_temp_checked(self):
+        t = self.inv_temp
+        if not (torch.is_tensor(t) and t.dtype == F64 and t.device == self.u.device and t.is_contiguous()
+                and t.numel() == self.n):
+            raise ValueError("inv_temp must be a contiguous float64 tensor of %d entries on %s" % (self.n, self.u.device))
+        return t
+
+    def swap(self, ladder_size, seed, round, replica, swap_counts, round_trips, inject_u=None):
+        """One replica-exchange round between adjacent rungs of the batch's ladders (ipmcmc_swap_replicas): the
+        batch is n / ladder_size ladders, ladder-major, tempered by `inv_temp`.  replica [n, 2] int32, swap_counts
+        [n_ladders, ladder_size - 1, 2] int64 and round_trips [n_ladders] int64 are updated in place; inject_u
+        [n_ladders, ladder_size - 1] replaces the Philox swap uniforms."""
+        K = int(ladder_size)
+        if K < 2 or self.n % K:
+            raise ValueError("%d chains do not form ladders of %d rungs" % (self.n, K))
+        L = self.n // K
+        for name, x, shape, dt in (("replica", replica, (self.n, 2), torch.int32),
+                                   ("swap_counts", swap_counts, (L, K - 1, 2), torch.int64),
+                                   ("round_trips", round_trips, (L,), torch.int64),
+                                   ("inject_u", inject_u, (L, K - 1), F64)):
+            if x is not None and (tuple(x.shape) != shape or x.dtype != dt or not x.is_contiguous()
+                                  or x.device != self.u.device):
+                raise ValueError("%s must be a contiguous %s tensor of shape %s on %s" % (name, dt, shape, self.u.device))
+        check(self.problem.lib.ipmcmc_swap_replicas(L, K, self.d, _ptr(self.u), _ptr(self.phi),
+                                                    _ptr(self._inv_temp_checked()), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                                    self.chain_offset, int(round), _ptr(inject_u), _ptr(replica),
+                                                    _ptr(swap_counts), _ptr(round_trips), _stream()))
         self.launches += 1
 
     def pooled(self):

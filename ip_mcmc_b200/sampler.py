@@ -22,6 +22,39 @@ from .potential import EvolutionPotential
 from .proposer import _GaussianStepProposer
 
 
+def run_recording(chains, spec, total, pre, sample_interval, trace, steps_per_launch=None, every=None,
+                  at_boundary=None):
+    """Advance a fresh `chains` by `total` steps, recording sample i of every chain into trace[:, i] (the step
+    accounting of MCMCSampler.run: `pre` unrecorded steps, then one sample every `sample_interval` steps).  One
+    launch unless it is cut: launches end every `steps_per_launch` steps and, when `every` is given, at every
+    multiple of `every` steps, after which at_boundary(step) runs.  A cut launch records into its own slice."""
+    def recorded_before(x):          # samples recorded by global steps < x
+        return max(0, x - pre) // sample_interval
+
+    done = 0
+    while True:
+        n = total - done
+        if steps_per_launch is not None:
+            n = min(n, steps_per_launch)
+        if every is not None:
+            n = min(n, every - done % every)
+        if n == total:
+            chains.run(spec, total, trace=trace)
+        else:
+            r0, r1 = recorded_before(done), recorded_before(done + n)
+            sub = None
+            if r1 > r0:
+                sub = torch.empty((chains.n, r1 - r0, chains.d), dtype=F64, device=trace.device)
+            chains.run(spec, n, trace=sub)
+            if sub is not None:
+                trace[:, r0:r1] = sub
+        done += n
+        if every is not None and done > 0 and done % every == 0:
+            at_boundary(done)
+        if done >= total:
+            return
+
+
 class MCMCSampler:
     def __init__(self, proposal, acceptance, rng):
         self.proposer = proposal
@@ -85,24 +118,7 @@ class MCMCSampler:
             raise ValueError("phi_0 is meaningless for a stateful forward model (Phi(u) is re-evaluated every step)")
         chains = ChainBatch(problem, u_0, n_chains=n_chains, chain_offset=chain_offset, scheduler=scheduler, phi0=phi_0)
         trace = torch.empty((chains.n, n_samples, chains.d), dtype=F64, device=problem.device)
-        if steps_per_launch is None or steps_per_launch >= total:
-            chains.run(spec, total, trace=trace)
-        else:
-            # chunked launches: each chunk records into its slice of the trace
-            def recorded_before(x):          # samples recorded by global steps < x
-                return max(0, x - pre) // sample_interval
-
-            done = 0
-            while done < total:
-                n = min(steps_per_launch, total - done)
-                r0, r1 = recorded_before(done), recorded_before(done + n)
-                sub = None
-                if r1 > r0:
-                    sub = torch.empty((chains.n, r1 - r0, chains.d), dtype=F64, device=problem.device)
-                chains.run(spec, n, trace=sub)
-                if sub is not None:
-                    trace[:, r0:r1] = sub
-                done += n
+        run_recording(chains, spec, total, pre, sample_interval, trace, steps_per_launch)
         pooled = chains.pooled()
         counters = chains.counters
         if pot.G.stateful and single:
