@@ -221,23 +221,20 @@ typedef struct ipmcmc_chain_buffers {
     /* optional IN: injected noise (parity mode; the reference's MockRNG seam)                  */
     const double *inject_w_dev; /* [n_chains, n_steps, d] proposal normals at the w level       */
     const double *inject_u_dev; /* [n_chains, n_steps]    accept uniforms                       */
-    /* optional scheduling hint (Burgers; results do not depend on it): the kernel runs
-       `warps_per_cta` chains per CTA (one warp each; 0 = library default) and warp w of CTA b
-       serves chain slot_chain_dev[b*warps_per_cta + w] (-1 = idle slot; NULL = identity).
-       Warps w and w+4 of a CTA share an SM sub-partition, so a caller that knows which chains
-       are expensive can pair heavy with light ones (ChainBatch does, from last launch's work). */
-    const int32_t *slot_chain_dev; /* [n_slots]                                                  */
-    int32_t n_slots;
-    int32_t warps_per_cta;
-    /* optional scratch of the DYNAMIC STEP SCHEDULER (Burgers with N <= 1024, where the work unit is a
-       chain, and Lorenz, where it is a warp's group of floor(32/K) chains; results do not depend on
-       it): int64 [sched_len >= 3*n_chains + 2], contents irrelevant on entry.  When given, persistent
-       warps take (chain, sched_chunk steps) work items from a FIFO of ready chains instead of a
-       fixed chain -> warp map, which keeps every SM sub-partition busy until the launch ends although
-       solve lengths are data dependent.  slot_chain_dev / warps_per_cta are then ignored.        */
+    /* reserved, ignored (formerly scheduling hints of a static chain -> warp map)                 */
+    const void *reserved_ptr0;
+    int32_t reserved0, reserved1;
+    /* scratch of the DYNAMIC STEP SCHEDULER, the only path of Burgers chains with N <= 1024 and d <= 32
+       (work unit: a chain) and of Lorenz chains (work unit: a warp's group of floor(32/K) chains): persistent
+       warps take (unit, sched_chunk steps) work items from a FIFO of ready units, which keeps every SM
+       sub-partition busy until the launch ends although solve lengths are data dependent.  Results do not
+       depend on it.  int64 [sched_len >= 3*units + 2], contents irrelevant on entry; NULL: the library
+       makes a stream-ordered allocation and frees it inside the call.  Ignored by the wide (d > 32) and
+       team (N > 1024) Burgers paths.                                                               */
     int64_t *sched_dev;
     int64_t sched_len;
-    int32_t sched_chunk;      /* Metropolis steps per work item (<=0: 1)                        */
+    int32_t sched_chunk;      /* Metropolis steps per work item (<= 0: Burgers min(4, max(1, n_steps/64)),
+                                 Lorenz 1)                                                          */
     int32_t reserved;
 } ipmcmc_chain_buffers;
 
@@ -358,7 +355,7 @@ typedef struct ipmcmc_host_io {
     double *phi_host;          /* OUT [n_chains] Phi(final state), or NULL                          */
     int64_t *counters_host;    /* OUT [n_chains, 6], or NULL                                        */
     double *pooled_host;       /* OUT [2d + 7] pooled moments + counters, or NULL                   */
-    int32_t scheduler;         /* 0: dynamic step scheduler where available (default), 1: static    */
+    int32_t reserved;          /* ignored (formerly the choice of a static scheduler)               */
     int32_t sched_chunk;       /* Metropolis steps per work item (<= 0: Burgers min(4, max(1, n_steps/64)), Lorenz 1) */
 } ipmcmc_host_io;
 

@@ -56,8 +56,8 @@ class ChainBuffers(C.Structure):
                 ("mom_count_dev", C.c_void_p), ("mom_mean_dev", C.c_void_p), ("mom_m2_dev", C.c_void_p),
                 ("counters_dev", C.c_void_p), ("trace_dev", C.c_void_p), ("n_record", C.c_int64),
                 ("steplog_dev", C.c_void_p), ("vlog_dev", C.c_void_p), ("inject_w_dev", C.c_void_p),
-                ("inject_u_dev", C.c_void_p), ("slot_chain_dev", C.c_void_p), ("n_slots", C.c_int32),
-                ("warps_per_cta", C.c_int32), ("sched_dev", C.c_void_p), ("sched_len", C.c_int64),
+                ("inject_u_dev", C.c_void_p), ("reserved_ptr0", C.c_void_p), ("reserved0", C.c_int32),
+                ("reserved1", C.c_int32), ("sched_dev", C.c_void_p), ("sched_len", C.c_int64),
                 ("sched_chunk", C.c_int32), ("reserved", C.c_int32)]
 
 
@@ -65,7 +65,7 @@ class HostIO(C.Structure):
     _fields_ = [("u0_host", c_double_p), ("phi0_host", c_double_p), ("model_state_host", c_double_p),
                 ("samples_host", c_double_p), ("n_record", C.c_int64), ("u_host", c_double_p),
                 ("phi_host", c_double_p), ("counters_host", c_int64_p), ("pooled_host", c_double_p),
-                ("scheduler", C.c_int32), ("sched_chunk", C.c_int32)]
+                ("reserved", C.c_int32), ("sched_chunk", C.c_int32)]
 
 
 # every symbol include/ipmcmc.h declares

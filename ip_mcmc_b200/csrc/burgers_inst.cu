@@ -14,9 +14,6 @@ namespace ipmcmc {
     template cudaError_t burgers_launch_forward<IPMCMC_TU_CPL, NUM, PAD>(const BurgersDev &, long long, const double *, \
                                                                          double *, double *, double *, long long *,  \
                                                                          cudaStream_t);                              \
-    template cudaError_t burgers_launch_chain<IPMCMC_TU_CPL, NUM, PAD>(const BurgersDev &, const SamplerDev &,          \
-                                                                       const ChainBufDev &, long long, long long, int, \
-                                                                       cudaStream_t);                                \
     template cudaError_t burgers_launch_chain_queue<IPMCMC_TU_CPL, NUM, PAD>(const BurgersDev &, const SamplerDev &,    \
                                                                              const ChainBufDev &, long long, long long, \
                                                                              int, cudaStream_t);                     \

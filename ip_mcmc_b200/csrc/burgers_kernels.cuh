@@ -1,19 +1,14 @@
-// Burgers kernels: batched forward evaluation and the fused Metropolis kernel.
-// One chain per warp, one warp per CTA (the hardware block scheduler then balances the
-// data-dependent solve lengths across the 148 SMs); the FV state never leaves registers, the end
-// state is staged once per solve in shared memory for the windowed trapezoid measurement.
+// Burgers kernels: batched forward evaluation and the fused Metropolis kernels.
+// One chain per warp up to 1024 cells: the chain kernel's persistent warps take work items from the step
+// queue (sched.cuh), which balances the data-dependent solve lengths across the SM sub-partitions; the wide
+// kernel (d > 32) maps chains onto warps statically.  One chain per CTA of 2 or 4 warps above 1024 cells (team
+// kernels).  The FV state never leaves registers; the end state is staged once per solve in shared memory
+// for the windowed trapezoid measurement.
 #pragma once
 #include "burgers.cuh"
 #include "burgers_team.cuh"
 #include "sampler.cuh"
 #include "sched.cuh"
-
-// Register budget of the static chain kernel: 128 registers (2 CTAs of 256 threads per SM) up to 8 cells
-// per lane, 255 from 16 cells per lane on, where 128 spill the state (measured: burgers_launch_impl.cuh,
-// burgers_launch_chain_queue).
-#ifndef IPMCMC_CHAIN_MINB
-#define IPMCMC_CHAIN_MINB(CPL) ((CPL) >= 16 ? 1 : 2)
-#endif
 
 namespace ipmcmc {
 
@@ -305,27 +300,6 @@ __device__ __forceinline__ void burgers_advance_chain(const SamplerDev &S, const
     for (long long s = s0; s < s1; ++s) metropolis_step(S, C, Gp, c, cg, s, n_steps, R, phi_of, true);
     burgers_store_chain<QUEUE>(S, C, Gp.lane, c, R);
     __syncwarp();
-}
-
-// W warps per CTA, one chain per warp.  Warps never synchronise with each other; the CTA shape
-// only pins which chains share an SM sub-partition (warp w -> SMSP w % 4).
-template <int CPL, int NUMERICS, bool PADDED>
-__global__ void __launch_bounds__(256, IPMCMC_CHAIN_MINB(CPL)) burgers_chain_kernel(const __grid_constant__ BurgersDev B,
-                                                            const __grid_constant__ SamplerDev S,
-                                                            const __grid_constant__ ChainBufDev C, long long n_chains,
-                                                            long long n_steps) {
-    extern __shared__ double smem_all[];
-    const int warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
-    double *smem = smem_all + (size_t)warp * (B.N + 2 * IPMCMC_MAX_OBS);
-    double *state = smem, *Gs = smem + B.N, *r2 = Gs + IPMCMC_MAX_OBS;
-    const Group Gp{0, 32, lane_id(), FULL};
-    const long long n_slots = C.slot_chain ? (long long)C.n_slots : n_chains;
-    for (long long slot = (long long)blockIdx.x * wpc + warp; slot < n_slots; slot += (long long)gridDim.x * wpc) {
-        const long long c = C.slot_chain ? (long long)C.slot_chain[slot] : slot;
-        if (c < 0 || c >= n_chains) continue;
-        burgers_advance_chain<false>(S, C, Gp, c, 0, n_steps, n_steps, LaneVec{},
-                                     BurgersPhiOf<CPL, NUMERICS, PADDED>{B, state, Gs, r2, Gp.lane});
-    }
 }
 
 // Dynamic step scheduler (sched.cuh): the work unit is a chain, an item is `chunk` Metropolis steps of it.

@@ -12,9 +12,6 @@ template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_forward(const BurgersDev &b, long long n, const double *u, double *G, double *phi,
                                    double *state, long long *work, cudaStream_t st);
 template <int CPL, int NUM, bool PAD>
-cudaError_t burgers_launch_chain(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,
-                                 long long n_steps, int wpc, cudaStream_t st);
-template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_chain_queue(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C,
                                        long long n_chains, long long n_steps, int chunk, cudaStream_t st);
 template <int CPL, int NUM, bool PAD>

@@ -35,14 +35,6 @@ cudaError_t burgers_launch_forward(const BurgersDev &b, long long n, const doubl
                   burgers_smem_bytes(b.N, wpc), st, b, n, u, G, phi, state, work);
 }
 
-template <int CPL, int NUM, bool PAD>
-cudaError_t burgers_launch_chain(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,
-                                long long n_steps, int wpc, cudaStream_t st) {
-    const long long slots = C.slot_chain ? (long long)C.n_slots : n_chains;
-    return launch(burgers_chain_kernel<CPL, NUM, PAD>, grid_for((slots + wpc - 1) / wpc), 32 * wpc,
-                  burgers_smem_bytes(b.N, wpc), st, b, S, C, n_chains, n_steps);
-}
-
 // Dynamic step scheduler (burgers_chain_queue_kernel): persistent warps, one wave.
 template <int CPL, int NUM, bool PAD>
 cudaError_t burgers_launch_chain_queue(const BurgersDev &b, const SamplerDev &S, const ChainBufDev &C, long long n_chains,

@@ -226,6 +226,20 @@ static int cu(cudaError_t e) {
     return 0;
 }
 
+// runs body(scratch) on the caller's scratch (checked against need) or a stream-ordered allocation
+template <class F>
+static int with_scratch(void *scratch, int64_t scratch_bytes, int64_t need, cudaStream_t st, const F &body) {
+    if (scratch) {
+        if (scratch_bytes < need) return fail(IPMCMC_EINVAL, "scratch: %lld bytes given, %lld needed", (long long)scratch_bytes, (long long)need);
+        return body(scratch);
+    }
+    void *tmp = nullptr;
+    CUDA_TRY(cudaMallocAsync(&tmp, (size_t)need, st));
+    const int rc = body(tmp);
+    cudaFreeAsync(tmp, st);
+    return rc;
+}
+
 #define BURGERS_TEAM_DISPATCH(FN, ...)                                                                  \
     do {                                                                                                \
         const bool fused = p->numerics == IPMCMC_NUMERICS_FUSED;                                        \
@@ -258,7 +272,7 @@ static int cu(cudaError_t e) {
 // CTA shape of the Lorenz kernels.  Batches that fit one wave get one CTA of W = ceil(warps / n_SM)
 // warps per SM, so that the warps of an SM are dealt round-robin onto its four sub-partitions
 // (warp w -> sub-partition w % 4); larger batches use 4-warp CTAs and the block scheduler.
-static int lorenz_warps_per_cta(long long warps, int K) {
+static int lorenz_cta_warps(long long warps, int K) {
     int n_sm = 148;
     sm_count(n_sm);
     int wpc = warps <= 8LL * n_sm ? (int)((warps + n_sm - 1) / n_sm) : 4;
@@ -306,7 +320,7 @@ extern "C" int ipmcmc_forward(ipmcmc_problem *p, int64_t n, const double *u_dev,
     if (!state_dev) return fail(IPMCMC_EINVAL, "Lorenz forward needs state_dev (carried initial condition)");
     const int groups = lorenz_groups(p->l.K);
     const long long warps = (n + groups - 1) / groups;
-    const int wpc = lorenz_warps_per_cta(warps, p->l.K);
+    const int wpc = lorenz_cta_warps(warps, p->l.K);
     LORENZ_DISPATCH(lorenz_forward_kernel, p->l.J, p->l.K, p->numerics,
                     <<<grid_for((warps + wpc - 1) / wpc), 32 * wpc, wpc * lorenz_smem_bytes(p->l.K), st>>>(
                         p->l, n, u_dev, G_dev, phi_dev, state_dev, (long long *)work_dev));
@@ -419,33 +433,29 @@ static int run_chains(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipm
     C.vlog = b->vlog_dev;
     C.inject_w = b->inject_w_dev;
     C.inject_u = b->inject_u_dev;
-    C.slot_chain = b->slot_chain_dev;
-    C.n_slots = b->n_slots;
-    C.sched = (long long *)b->sched_dev;
     C.inv_temp = inv_temp;
-    int chunk = b->sched_chunk > 0 ? b->sched_chunk : 1;   // steps per work item of the dynamic scheduler
-    if (const char *e = getenv("IPMCMC_SCHED_CHUNK")) chunk = atoi(e) > 0 ? atoi(e) : chunk;  // experiments
     if (p->model == IPMCMC_MODEL_BURGERS) {
-        int wpc = b->warps_per_cta > 0 ? b->warps_per_cta : 4;
-        if (wpc > 8) return fail(IPMCMC_EINVAL, "warps_per_cta=%d > 8", wpc);
-        if (b->slot_chain_dev && b->n_slots < 1) return fail(IPMCMC_EINVAL, "slot_chain_dev without n_slots");
         if (p->b.N > 1024) BURGERS_TEAM_DISPATCH(burgers_launch_team_chain, p->b, S, C, n_chains, n_steps, st);
         if (S.d > IPMCMC_MAX_DIM) BURGERS_DISPATCH(burgers_launch_wide_chain, p->b, S, C, n_chains, n_steps, st);
-        if (b->sched_dev) {
-            if (b->sched_len < sched_len(n_chains))
-                return fail(IPMCMC_EINVAL, "sched_len=%lld < 3*n_chains+2", (long long)b->sched_len);
-            if (n_chains >= (1LL << 31)) return fail(IPMCMC_EUNSUPPORTED, "dynamic scheduler: n_chains >= 2^31");
-            BURGERS_DISPATCH(burgers_launch_chain_queue, p->b, S, C, n_chains, n_steps, chunk, st);
-        }
-        BURGERS_DISPATCH(burgers_launch_chain, p->b, S, C, n_chains, n_steps, wpc, st);
+        if (n_chains >= (1LL << 31)) return fail(IPMCMC_EUNSUPPORTED, "dynamic scheduler: n_chains >= 2^31");
     }
-    const int groups = lorenz_groups(p->l.K);
-    const long long warps = (n_chains + groups - 1) / groups;
-    const int wpc = lorenz_warps_per_cta(warps, p->l.K);
-    if (b->sched_dev) {
-        // dynamic step scheduler over the warps' chain groups: persistent warps, one wave (255 registers:
-        // 8 warps per SM at most; the queue needs every launched CTA resident)
-        if (b->sched_len < sched_len(warps)) return fail(IPMCMC_EINVAL, "sched_len=%lld too short", (long long)b->sched_len);
+    // Every other chain runs on the dynamic step scheduler (sched.cuh), whose work unit is a Burgers chain or a warp's
+    // group of Lorenz chains.  Metropolis steps per work item: an item costs ~4 us of queue traffic and state reloads,
+    // so long Burgers launches use longer items (measured on B200, 1024 x 256 cells: +1 % at 200 steps per launch; 50
+    // steps: none).  A Lorenz item is two RK45 solves of a warp's chain group (~1.7 ms): one step per item balances best
+    // (4096 chains, 128 steps per launch: 1.87 M chain-steps/s against 1.83 M with two steps per item).
+    const bool lorenz = p->model == IPMCMC_MODEL_LORENZ;
+    const int groups = lorenz ? lorenz_groups(p->l.K) : 1;
+    const long long units = (n_chains + groups - 1) / groups;
+    int chunk = b->sched_chunk > 0 ? b->sched_chunk : lorenz ? 1 : (int)(n_steps / 64 < 1 ? 1 : (n_steps / 64 > 4 ? 4 : n_steps / 64));
+    if (const char *e = getenv("IPMCMC_SCHED_CHUNK")) chunk = atoi(e) > 0 ? atoi(e) : chunk;  // experiments
+    const int64_t sched_bytes = b->sched_dev ? b->sched_len * (int64_t)sizeof(int64_t) : 0;
+    return with_scratch(b->sched_dev, sched_bytes, sched_len(units) * (int64_t)sizeof(int64_t), st, [&](void *sched) {
+        C.sched = (long long *)sched;
+        if (!lorenz) BURGERS_DISPATCH(burgers_launch_chain_queue, p->b, S, C, n_chains, n_steps, chunk, st);
+        // Lorenz: persistent warps, one wave (255 registers: 8 warps per SM at most; the queue needs every launched CTA resident)
+        const long long warps = units;   // one warp per chain group
+        const int wpc = lorenz_cta_warps(warps, p->l.K);
         int n_sm = 148;
         CUDA_TRY(sm_count(n_sm));
         long long ctas;
@@ -466,11 +476,7 @@ static int run_chains(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipm
         LORENZ_DISPATCH(lorenz_chain_queue_kernel, p->l.J, p->l.K, p->numerics,
                         <<<(int)ctas, 32 * qwpc, qwpc * lorenz_smem_bytes(p->l.K), st>>>(p->l, S, C, n_chains, n_steps, chunk));
         return 0;
-    }
-    LORENZ_DISPATCH(lorenz_chain_kernel, p->l.J, p->l.K, p->numerics,
-                    <<<grid_for((warps + wpc - 1) / wpc), 32 * wpc, wpc * lorenz_smem_bytes(p->l.K), st>>>(
-                        p->l, S, C, n_chains, n_steps));
-    return 0;
+    });
 }
 
 extern "C" int ipmcmc_run(ipmcmc_problem *p, const ipmcmc_sampler_desc *s, const ipmcmc_chain_buffers *b,
@@ -668,20 +674,6 @@ extern "C" int64_t ipmcmc_diag_scratch_bytes(int64_t n_chains, int32_t dim, int6
     return (int64_t)((a > b ? a : b) * sizeof(double));
 }
 
-// runs body(scratch) on the caller's scratch (checked against need) or a stream-ordered allocation
-template <class F>
-static int with_scratch(void *scratch, int64_t scratch_bytes, int64_t need, cudaStream_t st, const F &body) {
-    if (scratch) {
-        if (scratch_bytes < need) return fail(IPMCMC_EINVAL, "diagnostics scratch: %lld bytes given, %lld needed", (long long)scratch_bytes, (long long)need);
-        return body(scratch);
-    }
-    void *tmp = nullptr;
-    CUDA_TRY(cudaMallocAsync(&tmp, (size_t)need, st));
-    const int rc = body(tmp);
-    cudaFreeAsync(tmp, st);
-    return rc;
-}
-
 extern "C" int ipmcmc_diag_tau(int64_t n_chains, int64_t n_draws, int32_t dim, const double *trace_dev, int64_t chain_stride,
                                double *tau_dev, void *stream) {
     if (int rc = diag_check(n_chains, n_draws, dim, trace_dev, chain_stride, 1)) return rc;
@@ -857,12 +849,11 @@ extern "C" int ipmcmc_sample_host(ipmcmc_problem *p, const ipmcmc_sampler_desc *
     const size_t B = (size_t)n_chains;
     const size_t nvar = p->model == IPMCMC_MODEL_LORENZ ? (size_t)p->l.nvar : 0;
     if (nvar && !io->model_state_host) return fail(IPMCMC_EINVAL, "Lorenz needs model_state_host");
-    const bool queue = io->scheduler == 0 && uses_queue(p);
     // one device arena: u | phi | count | mean | m2 | pooled | model_state | trace | counters | sched | pool scratch
     const size_t n_trace = io->samples_host ? B * (size_t)io->n_record * d : 0;
     const size_t n_dbl = B * d + B + B + B * d + B * d + (2 * d + 7) + B * nvar + n_trace;
     const size_t units = p->model == IPMCMC_MODEL_LORENZ ? (B + lorenz_groups(p->l.K) - 1) / lorenz_groups(p->l.K) : B;
-    const size_t n_sched = queue ? (size_t)sched_len((long long)units) : 0;
+    const size_t n_sched = uses_queue(p) ? (size_t)sched_len((long long)units) : 0;
     const size_t pool_bytes = (size_t)ipmcmc_pool_scratch_bytes(n_chains, d);
     double *arena = nullptr;
     cudaMemPool_t mem_pool = arena_pool();
@@ -903,13 +894,11 @@ extern "C" int ipmcmc_sample_host(ipmcmc_problem *p, const ipmcmc_sampler_desc *
     cb.counters_dev = (int64_t *)counters;
     cb.trace_dev = io->samples_host ? trace : nullptr;
     cb.n_record = io->samples_host ? io->n_record : 0;
-    if (queue) {   // the dynamic step scheduler, like ChainBatch (the fast path)
+    if (n_sched) {   // the step queue's scratch in the arena, as ChainBatch passes its own
         cb.sched_dev = (int64_t *)sched;
         cb.sched_len = (int64_t)n_sched;
-        // Metropolis steps per work item (engine.py, ChainBatch.run: same rule): a Lorenz item is already ~1.7 ms of solves
-        const int64_t auto_chunk = p->model == IPMCMC_MODEL_LORENZ ? 1 : (n_steps / 64 < 1 ? 1 : (n_steps / 64 > 4 ? 4 : n_steps / 64));
-        cb.sched_chunk = io->sched_chunk > 0 ? io->sched_chunk : (int32_t)auto_chunk;
     }
+    cb.sched_chunk = io->sched_chunk;
     rc = ipmcmc_run(p, s, &cb, n_chains, n_steps, stream);
     if (rc) return cleanup(rc);
     if (io->pooled_host) {

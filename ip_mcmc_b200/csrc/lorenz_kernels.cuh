@@ -1,5 +1,5 @@
 // Lorenz kernels: batched forward evaluation, the fused Metropolis kernel, and the RHS / single
-// RK-attempt probes used by the parity tests.  floor(32/K) chains per warp, one warp per CTA.
+// RK-attempt probes used by the parity tests.  floor(32/K) chains per warp.
 #pragma once
 #include "lorenz.cuh"
 #include "sampler.cuh"
@@ -100,8 +100,9 @@ __global__ void __launch_bounds__(256, 1) lorenz_forward_kernel(const __grid_con
 }
 
 // Metropolis steps [s0, s1) of the launch for the warp's group of chains c0 .. c0 + groups - 1
-// (chain c0 + slot on this lane group): load the chain state (ld_state<QUEUE>, sched.cuh), step, store it back.
-template <int J, int KT, int NUM, bool QUEUE>
+// (chain c0 + slot on this lane group): load the chain state, step, store it back.  Another SM may have
+// written the state earlier in the launch (sched.cuh): it is read and written through L2.
+template <int J, int KT, int NUM>
 __device__ __forceinline__ void lorenz_advance_group(const LorenzDev &P, const SamplerDev &Sd, const ChainBufDev &C,
                                                      const LorenzLanes<J, KT, NUM> &L, const Group &Gp, int slot,
                                                      double *Gs, double *r2, long long n_chains, long long n_steps,
@@ -117,18 +118,18 @@ __device__ __forceinline__ void lorenz_advance_group(const LorenzDev &P, const S
     for (int i = 0; i < J + 1; ++i) S.y[i] = 0.0;
     if (active) {
         const double *ms = C.model_state + c * P.nvar;
-        S.y[0] = ld_state<QUEUE>(ms + L.k);
+        S.y[0] = __ldcg(ms + L.k);
 #pragma unroll
-        for (int j = 0; j < J; ++j) S.y[1 + j] = ld_state<QUEUE>(ms + L.K + L.k * J + j);
+        for (int j = 0; j < J; ++j) S.y[1 + j] = __ldcg(ms + L.K + L.k * J + j);
     }
-    double ui = own ? ld_state<QUEUE>(C.u + c * d + L.k) : 0.0;
-    double phi_u = active ? ld_state<QUEUE>(C.phi + c) : 0.0;
+    double ui = own ? __ldcg(C.u + c * d + L.k) : 0.0;
+    double phi_u = active ? __ldcg(C.phi + c) : 0.0;
     long long cnt[CNT_N];
 #pragma unroll
     for (int k = 0; k < CNT_N; ++k) cnt[k] = 0;
     double reg_u = (Sd.accepter == IPMCMC_ACCEPT_RW) ? prior_regulariser(Sd, Gp, ui) : 0.0;
-    Welford mom{active ? ld_state<QUEUE>(C.mom_count + c) : 0.0, own ? ld_state<QUEUE>(C.mom_mean + c * d + L.k) : 0.0,
-                own ? ld_state<QUEUE>(C.mom_m2 + c * d + L.k) : 0.0};
+    Welford mom{active ? __ldcg(C.mom_count + c) : 0.0, own ? __ldcg(C.mom_mean + c * d + L.k) : 0.0,
+                own ? __ldcg(C.mom_m2 + c * d + L.k) : 0.0};
     long long n_rec = recorded_before(Sd, Sd.first_step + s0) - recorded_before(Sd, Sd.first_step);
 
     for (long long s = s0; s < s1; ++s) {
@@ -199,51 +200,30 @@ __device__ __forceinline__ void lorenz_advance_group(const LorenzDev &P, const S
     }
     if (active) {
         double *ms = C.model_state + c * P.nvar;
-        st_state<QUEUE>(ms + L.k, S.y[0]);
+        __stcg(ms + L.k, S.y[0]);
 #pragma unroll
-        for (int j = 0; j < J; ++j) st_state<QUEUE>(ms + L.K + L.k * J + j, S.y[1 + j]);
+        for (int j = 0; j < J; ++j) __stcg(ms + L.K + L.k * J + j, S.y[1 + j]);
         if (own) {
-            st_state<QUEUE>(C.u + c * d + L.k, ui);
-            st_state<QUEUE>(C.mom_mean + c * d + L.k, mom.mean);
-            st_state<QUEUE>(C.mom_m2 + c * d + L.k, mom.m2);
+            __stcg(C.u + c * d + L.k, ui);
+            __stcg(C.mom_mean + c * d + L.k, mom.mean);
+            __stcg(C.mom_m2 + c * d + L.k, mom.m2);
         }
         if (L.k == 0) {
-            st_state<QUEUE>(C.phi + c, phi_u);
-            st_state<QUEUE>(C.mom_count + c, mom.count);
+            __stcg(C.phi + c, phi_u);
+            __stcg(C.mom_count + c, mom.count);
             // a chain belongs to one warp at a time: read-modify-write through L2 needs no atomic
 #pragma unroll
             for (int k = 0; k < CNT_N; ++k)
-                st_state<QUEUE>(C.counters + c * CNT_N + k, ld_state<QUEUE>(C.counters + c * CNT_N + k) + cnt[k]);
+                __stcg(C.counters + c * CNT_N + k, __ldcg(C.counters + c * CNT_N + k) + cnt[k]);
         }
     }
     __syncwarp();
 }
 
-// Static chain -> warp map: warp w of the grid serves the groups w, w + n_warps, ...
-template <int J, int KT, int NUM>
-__global__ void __launch_bounds__(256, 1) lorenz_chain_kernel(const __grid_constant__ LorenzDev P,
-                                                          const __grid_constant__ SamplerDev Sd,
-                                                          const __grid_constant__ ChainBufDev C, long long n_chains,
-                                                          long long n_steps) {
-    extern __shared__ double smem_all[];
-    const int lane = lane_id();
-    const int groups = lorenz_groups(P.K);
-    const int warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
-    double *smem = smem_all + (size_t)warp * (lorenz_smem_bytes(P.K) / sizeof(double));
-    LorenzLanes<J, KT, NUM> L;
-    L.init(lane, P.K, groups);
-    const int slot = L.valid ? lane / P.K : groups;
-    double *Gs = smem + (size_t)slot * 2 * IPMCMC_MAX_OBS, *r2 = Gs + IPMCMC_MAX_OBS;
-    const Group Gp{L.base, P.K, L.k, FULL};
-    for (long long c0 = ((long long)blockIdx.x * wpc + warp) * groups; c0 < n_chains;
-         c0 += (long long)gridDim.x * wpc * groups)
-        lorenz_advance_group<J, KT, NUM, false>(P, Sd, C, L, Gp, slot, Gs, r2, n_chains, n_steps, c0, 0, n_steps);
-}
-
 // Dynamic step scheduler (sched.cuh): the work unit is a warp's group of floor(32/K) chains, an item is
 // `chunk` Metropolis steps of it.  With 820 warps on 592 sub-partitions (4096 chains, K = 6) a static map
 // leaves the sub-partitions that hold one warp idle for ~45 % of the launch; rotating the groups over the
-// warps lets every group advance at the average pace.  Bit-identical to the static kernel (tested).
+// warps lets every group advance at the average pace.
 template <int J, int KT, int NUM>
 __global__ void __launch_bounds__(256, 1) lorenz_chain_queue_kernel(const __grid_constant__ LorenzDev P,
                                                                 const __grid_constant__ SamplerDev Sd,
@@ -264,7 +244,7 @@ __global__ void __launch_bounds__(256, 1) lorenz_chain_queue_kernel(const __grid
     // the last rows leave at once instead of spinning on an empty queue beside a working warp
     if ((long long)warp * gridDim.x + blockIdx.x >= n_units) return;
     sched_serve(C.sched, n_units, n_steps, chunk, lane, [&](long long g, long long s0, long long s1) {
-        lorenz_advance_group<J, KT, NUM, true>(P, Sd, C, L, Gp, slot, Gs, r2, n_chains, n_steps, g * groups, s0, s1);
+        lorenz_advance_group<J, KT, NUM>(P, Sd, C, L, Gp, slot, Gs, r2, n_chains, n_steps, g * groups, s0, s1);
     });
 }
 

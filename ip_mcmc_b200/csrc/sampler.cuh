@@ -39,9 +39,7 @@ struct ChainBufDev {
     long long n_record;
     double *steplog, *vlog;
     const double *inject_w, *inject_u;
-    const int *slot_chain;
-    int n_slots;
-    long long *sched;   // dynamic step scheduler scratch (int64 [3*n_chains + 2]) or nullptr
+    long long *sched;   // step queue scratch (int64 [sched_len(work units)], sched.cuh); unused by the wide and team kernels
     const double *inv_temp;  // [n_chains] inverse temperature of each chain's likelihood, or nullptr (= 1)
 };
 

@@ -13,10 +13,11 @@ namespace ipmcmc {
 // memory: a chain is pushed back as soon as its item is done, so chains rotate over the warps,
 // advance at the same average pace and every warp stays busy until the queue runs dry.  The chain
 // state (u, Phi, moments: ~100 B) travels through L2 between items; Philox is keyed by (chain,
-// step), so the results do not depend on which warp ran which item (bit-identical to the static
-// kernel; tested).
+// step), so the results do not depend on which warp ran which item: the same bits for any chunk,
+// CTA shape and launch split (tests/test_gpu_chains.py, test_queue_is_pure_scheduling;
+// tests/test_gpu_lorenz.py, test_lorenz_queue_is_pure_scheduling).
 //
-// Scratch (caller-owned, int64): ring[cap] | progress[n] | head | tail, cap = 2*n (n = work units).
+// Scratch (int64, the caller's or a stream-ordered allocation of the library): ring[cap] | progress[n] | head | tail, cap = 2*n (n = work units).
 // Ring entry = ((lap+1) << 32) | chain for the ticket lap*cap + slot; 0 = consumed/empty.
 // ------------------------------------------------------------------------------------------------
 struct SchedView {

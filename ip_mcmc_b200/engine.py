@@ -5,7 +5,6 @@ There is no CPU path: constructing a Problem without a CUDA device or without th
 raises.
 """
 import ctypes as C
-import os
 
 import numpy as np
 import torch
@@ -127,55 +126,14 @@ class Problem:
         return dict(G=G, phi=phi, work=work, state=st)
 
 
-class Placement:
-    """Work-aware placement of chains on SM sub-partitions for SMALL batches (one wave).
-
-    With n <= 8 * n_SM chains the fused Burgers kernel runs one CTA of W = ceil(n / n_SM) warps per
-    SM, one chain per warp; warps w and w+4 of a CTA share a sub-partition (and its fp64 pipe).
-    Solve lengths are data dependent (FV steps ~ max|w| * N), so the launch lasts as long as the
-    most loaded sub-partition.  Before each launch the chains are ranked by the work they did in
-    the previous launch (a good predictor: states move slowly) and dealt out so that the heaviest
-    chains sit alone and the remaining heavy ones share with the lightest.  Pure scheduling: the
-    results do not depend on it (Philox is keyed by the chain id, not by the slot)."""
-
-    def __init__(self, n, n_sm, device):
-        self.W = min(8, -(-n // n_sm)) if n <= 8 * n_sm else 1
-        self.active = self.W > 4
-        if not self.active:
-            return
-        W, d = self.W, self.W - 4                      # d double bins (slots j, j+4), 4-d singles
-        n_cta = -(-n // W)
-        n_s, n_d = n_cta * (4 - d), n_cta * d
-        r = np.arange(n_cta * W)
-        slot = np.empty_like(r)
-        rs = r[:n_s]
-        slot[:n_s] = (rs // (4 - d)) * W + d + rs % (4 - d) if d < 4 else 0
-        b = np.arange(n_d)
-        slot[n_s:n_s + n_d] = (b // d) * W + b % d
-        b2 = n_d - 1 - b
-        slot[n_s + n_d:] = (b2 // d) * W + b2 % d + 4
-        assert np.array_equal(np.sort(slot), r)
-        self.n_slots = n_cta * W
-        self.slot_of_rank = torch.as_tensor(slot[:n], dtype=torch.int64).to(device)
-        self.slot_chain = torch.full((self.n_slots,), -1, dtype=torch.int32, device=device)
-
-    def update(self, work):
-        """work: cuda tensor [n] (any dtype) -- larger = more expensive."""
-        ranks = torch.argsort(work.to(torch.float64), descending=True)
-        self.slot_chain.fill_(-1)
-        self.slot_chain[self.slot_of_rank] = ranks.to(torch.int32)
-        return self.slot_chain
-
-
 class ChainBatch:
     """State of `n_chains` independent chains on the device (u, Phi(u), carried model state,
     Welford moments, counters)."""
 
     COUNTER_NAMES = ("calls", "accepts", "work_a", "work_b", "nonfinite", "constraint_rejects")
 
-    def __init__(self, problem, u0, n_chains=None, model_state=None, chain_offset=0, scheduler=None, phi0=None):
+    def __init__(self, problem, u0, n_chains=None, model_state=None, chain_offset=0, phi0=None):
         self.problem = problem
-        scheduler = scheduler or os.environ.get("IPMCMC_SCHEDULER", "dynamic")
         dev = problem.device
         d = problem.d
         u0 = np.asarray(u0, dtype=np.float64) if not torch.is_tensor(u0) else u0
@@ -227,26 +185,13 @@ class ChainBatch:
         self._keep = []
         self._pool_scratch = None
         self.launches = 0
-        self.placement = None
-        self._work_prev = None
         # optional [n_chains] float64 cuda tensor: inverse temperature of each chain's likelihood (replica
         # exchange, tempering.py); None runs the untempered kernel path (ipmcmc_run)
         self.inv_temp = None
-        self.sched = None          # scratch of the dynamic step scheduler (Burgers N <= 1024, Lorenz)
+        self.sched = None          # scratch of the dynamic step scheduler (Burgers N <= 1024 and d <= 32, Lorenz)
         self.sched_chunk = 0       # Metropolis steps per work item; 0 = automatic (Burgers: min(4, max(1, n_steps // 64)); Lorenz: 1)
-        if problem.kind == _lib.MODEL_LORENZ:
-            if scheduler == "dynamic":
-                self.sched = torch.empty((3 * self.n + 2,), dtype=torch.int64, device=dev)
-            elif scheduler != "static":
-                raise ValueError("scheduler must be 'dynamic' or 'static'")
-        if problem.kind == _lib.MODEL_BURGERS:
-            n_sm = torch.cuda.get_device_properties(dev).multi_processor_count
-            if scheduler == "dynamic" and problem.model.N <= 1024 and d <= _lib.MAX_DIM:
-                self.sched = torch.empty((3 * self.n + 2,), dtype=torch.int64, device=dev)
-            elif scheduler not in ("dynamic", "static"):
-                raise ValueError("scheduler must be 'dynamic' or 'static'")
-            else:
-                self.placement = Placement(self.n, n_sm, dev)
+        if problem.kind == _lib.MODEL_LORENZ or (problem.model.N <= 1024 and d <= _lib.MAX_DIM):
+            self.sched = torch.empty((3 * self.n + 2,), dtype=torch.int64, device=dev)
 
     def run(self, spec, n_steps, trace=None, steplog=None, vlog=None, inject_w=None, inject_u=None):
         """Advance all chains by n_steps in ONE launch of the fused kernel (ipmcmc_run).
@@ -270,21 +215,7 @@ class ChainBatch:
         if self.sched is not None:
             b.sched_dev = _ptr(self.sched)
             b.sched_len = self.sched.numel()
-            # a work item costs ~4 us of queue traffic and state reloads: long Burgers launches use longer
-            # items (measured on B200, 1024 x 256 cells: +1 % at 200 steps per launch; 50 steps: none).  A Lorenz
-            # item is two RK45 solves of a warp's chain group (~1.7 ms): one step per item balances best
-            # (4096 chains, 128 steps per launch: 1.87 M chain-steps/s against 1.83 M with two steps per item)
-            auto = 1 if self.problem.kind == _lib.MODEL_LORENZ else min(4, max(1, int(n_steps) // 64))
-            b.sched_chunk = self.sched_chunk or auto
-        pl = self.placement
-        if pl is not None:
-            b.warps_per_cta = pl.W
-            if pl.active and self._work_prev is not None:
-                table = pl.update(self.counters[:, 2] - self._work_prev)
-                b.slot_chain_dev = _ptr(table)
-                b.n_slots = pl.n_slots
-            if pl.active:
-                self._work_prev = self.counters[:, 2].clone()
+        b.sched_chunk = self.sched_chunk
         if self.inv_temp is None:
             check(lib.ipmcmc_run(self.problem.handle, C.byref(s), C.byref(b), self.n, int(n_steps), _stream()))
         else:

@@ -90,7 +90,7 @@ class MCMCSampler:
         return spec, pot, a
 
     def run(self, u_0, n_samples, burn_in=1000, sample_interval=200, n_chains=None, chain_offset=0,
-            steps_per_launch=None, return_device=False, recompute_phi_u=None, scheduler=None, out=None, phi_0=None, diagnostics=False):
+            steps_per_launch=None, return_device=False, recompute_phi_u=None, out=None, phi_0=None, diagnostics=False):
         """Same step accounting as the reference (sampler.py:18-28): max(0, burn_in - interval)
         unrecorded steps, then n_samples * interval steps recording every interval-th state.
 
@@ -116,7 +116,7 @@ class MCMCSampler:
         single = n_chains is None and np.ndim(u_0) == 1
         if phi_0 is not None and pot.G.stateful:
             raise ValueError("phi_0 is meaningless for a stateful forward model (Phi(u) is re-evaluated every step)")
-        chains = ChainBatch(problem, u_0, n_chains=n_chains, chain_offset=chain_offset, scheduler=scheduler, phi0=phi_0)
+        chains = ChainBatch(problem, u_0, n_chains=n_chains, chain_offset=chain_offset, phi0=phi_0)
         trace = torch.empty((chains.n, n_samples, chains.d), dtype=F64, device=problem.device)
         run_recording(chains, spec, total, pre, sample_interval, trace, steps_per_launch)
         pooled = chains.pooled()
@@ -150,7 +150,7 @@ class MCMCSampler:
         return res[0] if single else res
 
     def run_host(self, u_0, n_samples, burn_in=1000, sample_interval=200, n_chains=None, chain_offset=0,
-                 recompute_phi_u=None, out=None, phi_0=None, scheduler="dynamic"):
+                 recompute_phi_u=None, out=None, phi_0=None):
         """`run` through the C entry point `ipmcmc_sample_host` alone: NumPy (host) buffers in and out,
         every copy and the device arena inside the C call, no torch tensor anywhere on the path -- what a
         binding from another language would execute.  Same step accounting and results as `run` (tested
@@ -200,7 +200,6 @@ class MCMCSampler:
         io.samples_host, io.n_record = _lib.as_double_p(out), n_samples
         io.u_host, io.phi_host = _lib.as_double_p(u_end), _lib.as_double_p(phi_end)
         io.counters_host, io.pooled_host = counters.ctypes.data_as(_lib.c_int64_p), _lib.as_double_p(pooled)
-        io.scheduler = 0 if scheduler == "dynamic" else 1
         _lib.check(problem.lib.ipmcmc_sample_host(problem.handle, C.byref(desc), B, total, C.byref(io), None))
         if ms is not None and single:
             pot.G.IC = ms[0]

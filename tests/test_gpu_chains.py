@@ -219,25 +219,24 @@ def test_free_running_chain_statistics_vs_cpu_oracle(G):
 
 def test_host_buffer_entry_point_matches_device_path(G):
     """ipmcmc_sample_host (host pointers in/out, copies inside; MCMCSampler.run_host) == MCMCSampler.run on
-    the same seed -- samples, counters, pooled moments, final states -- with the dynamic scheduler and the
-    static map, and continued from a known Phi(u_0) without the extra solve."""
+    the same seed -- samples, counters, pooled moments, final states -- and continued from a known Phi(u_0)
+    without the extra solve."""
     import ip_mcmc_b200 as M
     f, pot, prior, _ = G.burgers_setup(32, "fused")
     mk = lambda: M.MCMCSampler(M.ConstSteppCNProposer(0.25, prior), M.CountedAccepter(M.pCNAccepter(pot)), np.random.default_rng(4))
     n_chains, n = 9, 25
     s = mk()
     ref = s.run(np.zeros(3), n, 0, 1, n_chains=n_chains)
-    for sched in ("dynamic", "static"):
-        h = mk()
-        got = h.run_host(np.zeros(3), n, 0, 1, n_chains=n_chains, scheduler=sched)
-        assert h.last_run["seed"] == s.last_run["seed"]
-        assert np.array_equal(got, ref)
-        assert np.array_equal(h.last_run["per_chain_counters"], s.last_run["per_chain_counters"].cpu().numpy())
-        assert h.accepter.calls == n_chains * n and h.accepter.accepts == s.accepter.accepts
-        assert h.last_run["pooled_count"] == n_chains * n
-        np.testing.assert_allclose(h.last_run["pooled_mean"], ref.reshape(-1, 3).mean(0), rtol=1e-12)
-        np.testing.assert_allclose(h.last_run["pooled_var"], ref.reshape(-1, 3).var(0, ddof=1), rtol=1e-10)
-        assert np.array_equal(h.last_run["u"], ref[:, -1]) and np.array_equal(h.last_run["phi"], s.last_run["phi"].cpu().numpy())
+    h = mk()
+    got = h.run_host(np.zeros(3), n, 0, 1, n_chains=n_chains)
+    assert h.last_run["seed"] == s.last_run["seed"]
+    assert np.array_equal(got, ref)
+    assert np.array_equal(h.last_run["per_chain_counters"], s.last_run["per_chain_counters"].cpu().numpy())
+    assert h.accepter.calls == n_chains * n and h.accepter.accepts == s.accepter.accepts
+    assert h.last_run["pooled_count"] == n_chains * n
+    np.testing.assert_allclose(h.last_run["pooled_mean"], ref.reshape(-1, 3).mean(0), rtol=1e-12)
+    np.testing.assert_allclose(h.last_run["pooled_var"], ref.reshape(-1, 3).var(0, ddof=1), rtol=1e-10)
+    assert np.array_equal(h.last_run["u"], ref[:, -1]) and np.array_equal(h.last_run["phi"], s.last_run["phi"].cpu().numpy())
     # continuation with a known Phi(u_0): one solve per step, none for u_0; same as the device path
     a, b = mk(), mk()
     ra = a.run(s.last_run["u"], 10, 0, 1, phi_0=s.last_run["phi"])
@@ -249,43 +248,52 @@ def test_host_buffer_entry_point_matches_device_path(G):
     assert np.array_equal(rc, ra) and c.last_run["counters"]["work_b"] == n_chains * 11
 
 
-def test_placement_does_not_change_results(G):
-    """The work-aware slot table is pure scheduling: one-wave batches (placement active) give the
-    same chains as the same chains run inside a larger batch (placement inactive)."""
-    import ip_mcmc_b200 as M
-    import torch
-    f, pot, prior, _ = G.burgers_setup(32)
-    n_sm = torch.cuda.get_device_properties(0).multi_processor_count
-    n = 5 * n_sm + 3                      # W = 6 warps per CTA -> placement active
-    mk = lambda: M.MCMCSampler(M.ConstSteppCNProposer(0.25, prior), M.pCNAccepter(pot), np.random.default_rng(8))
-    a = mk()
-    out_a = a.run(np.zeros(3), 12, 0, 1, n_chains=n, steps_per_launch=4, scheduler="static")   # 3 launches: table used from the 2nd
-    assert a.last_run["chains"].placement.active
-    b = mk()
-    out_b = b.run(np.zeros(3), 12, 0, 1, n_chains=9 * n_sm, scheduler="static")                # > 8 n_SM: no placement
-    assert not b.last_run["chains"].placement.active
-    assert np.array_equal(out_a, out_b[:n])
-
-
 @pytest.mark.parametrize("N,n_chains,steps_per_launch", [(32, 700, None), (64, 1500, 5), (256, 1024, 7), (100, 333, 3)])
-def test_dynamic_scheduler_bit_identical_to_static(G, N, n_chains, steps_per_launch):
-    """The dynamic step scheduler (persistent warps + FIFO of ready chains, chain state travelling
-    through L2 between work items) is pure scheduling: samples, per-chain counters and Welford
-    moments equal the static one-chain-per-warp kernel bit for bit (small batch, > 8 n_SM batch,
-    the bench shape, a padded grid)."""
+def test_queue_is_pure_scheduling(G, N, n_chains, steps_per_launch, monkeypatch):
+    """The dynamic step scheduler (persistent warps + FIFO of ready chains, chain state travelling through L2
+    between work items) is pure scheduling: samples, per-chain counters and Welford moments are the same bits
+    with the default work items (4 steps for a 262-step launch) and CTA shape in one launch, and with one step
+    per item, one warp per SM when the batch is one wave (148 warps serve hundreds of chains, which change warps
+    at almost every step) and the launch split (small batch, > 8 n_SM batch, the bench shape, a padded grid)."""
     import ip_mcmc_b200 as M
     f, pot, prior, _ = G.burgers_setup(N, "fused")
     mk = lambda: M.MCMCSampler(M.ConstSteppCNProposer(0.25, prior), M.CountedAccepter(M.pCNAccepter(pot)),
                                np.random.default_rng(8))
     a, b = mk(), mk()
-    out_a = a.run(np.zeros(3), 10, 4, 2, n_chains=n_chains, steps_per_launch=steps_per_launch, scheduler="static")
-    out_b = b.run(np.zeros(3), 10, 4, 2, n_chains=n_chains, steps_per_launch=steps_per_launch, scheduler="dynamic")
+    out_a = a.run(np.zeros(3), 130, 4, 2, n_chains=n_chains)
+    monkeypatch.setenv("IPMCMC_SCHED_CHUNK", "1")
+    monkeypatch.setenv("IPMCMC_SCHED_WPC", "1")          # read for one-wave batches (<= 8 n_SM chains) only
+    out_b = b.run(np.zeros(3), 130, 4, 2, n_chains=n_chains, steps_per_launch=steps_per_launch)
     ca, cb = a.last_run["chains"], b.last_run["chains"]
-    assert ca.sched is None and cb.sched is not None
+    assert ca.sched is not None and cb.sched is not None
     assert np.array_equal(out_a, out_b)
     assert torch.equal(ca.counters, cb.counters) and torch.equal(ca.u, cb.u) and torch.equal(ca.phi, cb.phi)
     assert torch.equal(ca.mom_count, cb.mom_count) and torch.equal(ca.mom_mean, cb.mom_mean) and torch.equal(ca.mom_m2, cb.mom_m2)
     assert a.accepter.calls == b.accepter.calls and a.accepter.accepts == b.accepter.accepts
+
+
+def test_library_allocates_queue_scratch(G):
+    """ipmcmc_run without scheduler scratch (sched_dev = NULL) runs the queue on a stream-ordered allocation of the
+    library's: the same bits as with ChainBatch's scratch, over two launches."""
+    import ip_mcmc_b200 as M
+    from ip_mcmc_b200 import _lib
+    f, pot, prior, _ = G.burgers_setup(64, "fused")
+    spec = M.SamplerSpec(3, _lib.PROPOSE_PCN, _lib.ACCEPT_PCN, coef_u=np.sqrt(1 - 0.25 ** 2), coef_w=0.25,
+                         factor=np.full(3, 0.25), seed=11)
+    runs = []
+    for own in (True, False):
+        ch = M.ChainBatch(pot.problem(), np.zeros(3), n_chains=300)
+        assert ch.sched is not None
+        if not own:
+            ch.sched = None
+        traces = [torch.empty((300, 20, 3), dtype=torch.float64, device="cuda") for _ in range(2)]
+        for t in traces:
+            ch.run(spec, 20, trace=t)
+        runs.append((torch.cat(traces, 1), ch))
+    (ta, ca), (tb, cb) = runs
+    assert torch.equal(ta, tb) and ca.counters[:, 1].sum().item() > 0
+    for name in ("u", "phi", "counters", "mom_count", "mom_mean", "mom_m2"):
+        assert torch.equal(getattr(ca, name), getattr(cb, name)), name
 
 
 def test_grid_refinement_study_driver(G):

@@ -218,25 +218,49 @@ def test_lorenz_chain_first_steps_and_statistics(G):
 
 
 @pytest.mark.parametrize("n_chains,n_samples,steps_per_launch", [(33, 6, None), (1003, 5, 2), (7, 4, 3)])
-def test_lorenz_dynamic_scheduler_bit_identical_to_static(G, n_chains, n_samples, steps_per_launch):
+def test_lorenz_queue_is_pure_scheduling(G, n_chains, n_samples, steps_per_launch, monkeypatch):
     """The dynamic step scheduler of the Lorenz kernel (work unit = a warp's group of 5 chains, the carried
     initial condition travelling through L2 between work items) is pure scheduling: samples, carried
-    states, counters and moments equal the static kernel bit for bit (ragged last group, several launches,
-    more groups than SMs)."""
+    states, counters and moments are the same bits with one step per work item in one launch and with three
+    steps per item over the launch split (ragged last group, several launches, more groups than SMs)."""
     import ip_mcmc_b200 as M
     f, pot, prior, p = _lorenz_setup(0.5, numerics="fused")
     mk = lambda: M.MCMCSampler(M.ConstStepStandardRWProposer(0.125, prior),
                                M.CountedAccepter(M.StandardRWAccepter(pot, prior)), np.random.default_rng(5))
     a, b = mk(), mk()
-    out_a = a.run(p["u0"], n_samples, 2, 1, n_chains=n_chains, steps_per_launch=steps_per_launch, scheduler="static")
-    out_b = b.run(p["u0"], n_samples, 2, 1, n_chains=n_chains, steps_per_launch=steps_per_launch, scheduler="dynamic")
+    out_a = a.run(p["u0"], n_samples, 2, 1, n_chains=n_chains)
+    monkeypatch.setenv("IPMCMC_SCHED_CHUNK", "3")
+    out_b = b.run(p["u0"], n_samples, 2, 1, n_chains=n_chains, steps_per_launch=steps_per_launch)
     ca, cb = a.last_run["chains"], b.last_run["chains"]
-    assert ca.sched is None and cb.sched is not None
+    assert ca.sched is not None and cb.sched is not None
     assert np.array_equal(out_a, out_b)
     assert torch.equal(ca.model_state, cb.model_state)
     assert torch.equal(ca.counters, cb.counters) and torch.equal(ca.u, cb.u) and torch.equal(ca.phi, cb.phi)
     assert torch.equal(ca.mom_count, cb.mom_count) and torch.equal(ca.mom_mean, cb.mom_mean) and torch.equal(ca.mom_m2, cb.mom_m2)
     assert a.accepter.calls == b.accepter.calls and a.accepter.accepts == b.accepter.accepts
+
+
+def test_lorenz_library_allocates_queue_scratch(G):
+    """ipmcmc_run without scheduler scratch (sched_dev = NULL) on Lorenz chains: the same bits, carried states
+    included, as with ChainBatch's scratch."""
+    import ip_mcmc_b200 as M
+    from ip_mcmc_b200 import _lib
+    f, pot, prior, p = _lorenz_setup(0.5, numerics="fused")
+    spec = M.SamplerSpec(3, _lib.PROPOSE_RW, _lib.ACCEPT_RW, coef_u=1.0, coef_w=0.5, factor=np.sqrt([10., 1, 10]),
+                         prior_chol=prior.L, recompute_phi_u=True, seed=11)
+    runs = []
+    for own in (True, False):
+        ch = M.ChainBatch(pot.problem(), p["u0"], n_chains=23)
+        assert ch.sched is not None
+        if not own:
+            ch.sched = None
+        trace = torch.empty((23, 4, 3), dtype=torch.float64, device="cuda")
+        ch.run(spec, 4, trace=trace)
+        runs.append((trace, ch))
+    (ta, ca), (tb, cb) = runs
+    assert torch.equal(ta, tb)
+    for name in ("model_state", "u", "phi", "counters", "mom_count", "mom_mean", "mom_m2"):
+        assert torch.equal(getattr(ca, name), getattr(cb, name)), name
 
 
 @pytest.mark.parametrize("numerics", ["exact", "fused"])

@@ -51,9 +51,9 @@ def _problem(G, N, numerics, d):
     return M.EvolutionPotential(f, f.at_parameters(truth), M.GaussianDistribution(np.zeros(5), G.NOISE_COV))
 
 
-def _run_batch(pot, spec, n_chains, n_steps, inv_temp, u0, scheduler=None):
+def _run_batch(pot, spec, n_chains, n_steps, inv_temp, u0):
     import ip_mcmc_b200 as M
-    ch = M.ChainBatch(pot.problem(), u0, n_chains=n_chains, scheduler=scheduler)
+    ch = M.ChainBatch(pot.problem(), u0, n_chains=n_chains)
     if inv_temp is not None:
         ch.inv_temp = torch.as_tensor(inv_temp, dtype=torch.float64).cuda().contiguous()
     trace = torch.empty((n_chains, n_steps, ch.d), dtype=torch.float64, device="cuda")
@@ -61,24 +61,24 @@ def _run_batch(pot, spec, n_chains, n_steps, inv_temp, u0, scheduler=None):
     return trace, ch
 
 
-@pytest.mark.parametrize("N,numerics,d,kind,scheduler", [
-    (256, "fused", 3, "pcn", "dynamic"),     # the bench shape
-    (64, "exact", 3, "pcn", "dynamic"),
-    (64, "exact", 3, "rw", "static"),
-    (64, "fused", 3, "boxrw", "dynamic"),
-    (2048, "fused", 3, "pcn", None),          # team solver
-    (64, "fused", 33, "pcn", None),           # wide path
-    (64, "exact", 33, "boxrw", None),
+@pytest.mark.parametrize("N,numerics,d,kind", [
+    (256, "fused", 3, "pcn"),     # the bench shape
+    (64, "exact", 3, "pcn"),
+    (64, "exact", 3, "rw"),
+    (64, "fused", 3, "boxrw"),
+    (2048, "fused", 3, "pcn"),    # team solver
+    (64, "fused", 33, "pcn"),     # wide path
+    (64, "exact", 33, "boxrw"),
 ])
-def test_unit_inverse_temperature_is_ipmcmc_run(G, N, numerics, d, kind, scheduler):
+def test_unit_inverse_temperature_is_ipmcmc_run(G, N, numerics, d, kind):
     """ipmcmc_run_tempered with t = 1 everywhere: the same bits as ipmcmc_run in samples, u, Phi, counters, moments."""
     pot = _problem(G, N, numerics, d)
     spec = {"pcn": _pcn_spec, "rw": _rw_spec, "boxrw": lambda d: _rw_spec(d, box=True)}[kind](d)
     spec.seed = 1234
     n, steps = (16 if N > 1024 else 96), (6 if N > 1024 else 30)
     u0 = np.zeros(d)
-    t0, c0 = _run_batch(pot, spec, n, steps, None, u0, scheduler)
-    t1, c1 = _run_batch(pot, spec, n, steps, np.ones(n), u0, scheduler)
+    t0, c0 = _run_batch(pot, spec, n, steps, None, u0)
+    t1, c1 = _run_batch(pot, spec, n, steps, np.ones(n), u0)
     assert torch.equal(t0, t1)
     for name in ("u", "mom_count", "mom_mean", "mom_m2", "counters"):
         assert torch.equal(getattr(c0, name), getattr(c1, name)), name

@@ -12,9 +12,8 @@ prior = M.GaussianDistribution(PM, 0.25 ** 2 * np.identity(3))
 for N, num in ((64, "fused"), (100, "exact"), (256, "fused")):
     f = M.BurgersFVM(N=N, numerics=num)
     pot = M.EvolutionPotential(f, f.at_parameters(TRUTH), noise)
-    for sched in ("dynamic", "static"):
-        s = M.MCMCSampler(M.ConstSteppCNProposer(0.25, prior), M.CountedAccepter(M.pCNAccepter(pot)), np.random.default_rng(1))
-        out = s.run(np.zeros(3), 6, 0, 1, n_chains=37, scheduler=sched)
+    s = M.MCMCSampler(M.ConstSteppCNProposer(0.25, prior), M.CountedAccepter(M.pCNAccepter(pot)), np.random.default_rng(1))
+    out = s.run(np.zeros(3), 6, 0, 1, n_chains=37)
     h = M.MCMCSampler(M.ConstStepStandardRWProposer(0.01, prior), M.CountedAccepter(M.StandardRWAccepter(pot, prior)), np.random.default_rng(1))
     h.run_host(np.zeros(3), 5, 0, 1, n_chains=11)
 print("burgers ok")
@@ -36,9 +35,8 @@ for num in ("fused", "exact"):
     fl = M.Lorenz96Moments(6, 4, 0.25, 1.0, g["prior_means"], g["IC"], numerics=num)
     pl = M.EvolutionPotential(fl, g["y"], M.GaussianDistribution(np.zeros(30), 0.25 * np.diag(g["var"])))
     pr = M.GaussianDistribution(np.zeros(3), np.diag([10., 1, 10]))
-    for sched in ("dynamic", "static"):
-        M.MCMCSampler(M.ConstStepStandardRWProposer(0.125, pr), M.CountedAccepter(M.StandardRWAccepter(pl, pr)),
-                      np.random.default_rng(1)).run(g["u0"], 3, 0, 1, n_chains=13, scheduler=sched)
+    M.MCMCSampler(M.ConstStepStandardRWProposer(0.125, pr), M.CountedAccepter(M.StandardRWAccepter(pl, pr)),
+                  np.random.default_rng(1)).run(g["u0"], 3, 0, 1, n_chains=13)
 print("lorenz ok")
 r = studies.chain_length_study(chain_length=200, n_chains=3, N=32, sample_interval=5, steps_per_launch=70)
 print("study ok", r["counts"].sum())
